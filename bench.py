@@ -2,12 +2,15 @@
 """bench.py - TRPL forward simulations per second (nx=128, FP64), BASELINE.json's metric.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--sets S]
+                    [--dump-outputs DIR]
 
 Workload (config.workload): BASELINE configs[1] - 4096 random parameter sets (log-uniform in the
 prior box of the reference's Inputs/mcmc0.txt, as Dense_Sample/dense_sampling.py:17-35 draws them)
 x the 6 TRPL curves of the staub_MAPI_threepower_twothick example (nx=128, 119 measurement times
 each), 'std' model, PER GPU (weak scaling: every rank evaluates its own 4096 sets).  One "step" is
-one pass of the hot path over that batch: 24576 forward simulations + likelihoods.
+one pass of the hot path over that batch: 24576 forward simulations + likelihoods.  The parameter
+sets are drawn from fixed seeds and the measurement is stored (tests/golden/bench_measurement.npz),
+so the inputs are the same from run to run and from build to build.
 
 value   device-timed throughput, inputs resident in HBM (CUDA events on the library's stream)
 e2e     the same through the public API with HOST numpy buffers (H2D + kernel + D2H inside)
@@ -238,14 +241,30 @@ def barrier(dist, local):
         torch.cuda.synchronize(local)
 
 
-def synth_measurement(ctx_eval, ini, t, rng):
-    """Measurement = simulated curves of the initial guess, log10, renoised (like staub's renoised file)."""
-    sf = make_shared_fields(ini, t, [np.zeros(len(t))] * 6, [np.ones(len(t))] * 6)
-    res = ctx_eval(GUESS[None, :], np.ones(1), {"TRPL": SIGMA}, sf, want_curves=True)
-    cur = res.curves.reshape(6, len(t))
-    vals = [np.log10(cur[m]) + 0.02 * rng.standard_normal(len(t)) for m in range(6)]
-    uncs = [np.full(len(t), 0.02) for _ in range(6)]
-    return vals, uncs
+def workload_measurement():
+    """Measurement = simulated curves of the initial guess, log10, renoised (like staub's renoised
+    file): this project's kernel at rtol 1e-7, plus 0.02 x default_rng(1234).standard_normal per
+    curve; uncertainty 0.02.  It is stored rather than simulated at start-up, so that what a build
+    is given does not depend on that build's own arithmetic."""
+    g = np.load(os.path.join(ROOT, "tests", "golden", "bench_measurement.npz"))
+    return list(g["vals"]), list(g["uncs"])
+
+
+DUMP_LIMIT_BYTES = 60 << 20    # array data; with the .npy headers a dump stays under 64 MB
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each [n_sets, ...] array as out_dir/<name>.npy in float64, plus set_index.npy: the
+    parameter sets the rows belong to.  That is every set, or a fixed, seeded sample of them when
+    every set would exceed DUMP_LIMIT_BYTES."""
+    n_sets = len(next(iter(arrays.values())))
+    row_bytes = 8 * (1 + sum(a[0].size for a in arrays.values()))
+    keep = np.arange(n_sets)
+    if n_sets * row_bytes > DUMP_LIMIT_BYTES:
+        keep = np.sort(np.random.default_rng(0).choice(n_sets, DUMP_LIMIT_BYTES // row_bytes, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in dict(arrays, set_index=np.arange(n_sets)).items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.asarray(a, dtype=np.float64)[keep])
 
 
 def run_ours(args):
@@ -257,8 +276,7 @@ def run_ours(args):
     ini, t = workload_inputs()
     ctx = get_context(local)
     info = ctx.device_info()
-    rng = np.random.default_rng(1234)
-    vals, uncs = synth_measurement(lambda *a, **k: tme.eval_trial_moves(*a, cache=None, **k), ini, t, rng)
+    vals, uncs = workload_measurement()
     sf = make_shared_fields(ini, t, vals, uncs)
     cache = tme.PathCache(sf, device=local)
     states = draw_states(args.sets, seed=20261018 + rank)        # every rank its own shard
@@ -374,6 +392,9 @@ def run_ours(args):
                   "kernel_ms_each": [float(x) for x in kernel_ms],
                   "per_rank_[step_ms,kernel_ms,integrator_steps]": per_rank},
     }
+    if args.dump_outputs:
+        # what a caller of the timed path receives from its last step (Context.download)
+        dump_outputs(args.dump_outputs, {"logll": ll, "status": status, "nsteps": nsteps})
     print(json.dumps(out), flush=True)
     if dist is not None:
         dist.destroy_process_group()
@@ -593,7 +614,13 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip the configs[2], [3], [4] segments")
     ap.add_argument("--pt-iters", type=int, default=41)
     ap.add_argument("--dense-points", type=int, default=65536, help="dense-grid points per GPU")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed for rank 0's parameter sets "
+                         "as DIR/<name>.npy (float64): logll [set, curve, temperature slot], status [set, curve], "
+                         "nsteps [set, curve, accepted|rejected], set_index [set]")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the GPU path's outputs (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -1,14 +1,12 @@
 import sys, os, time, json
-sys.path.insert(0, '/root/repo')
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
 import bench
 from metrotrpl_b200 import dense_sampling as ds, _capi
-from metrotrpl_b200 import trial_move_evaluation as tme
 from metrotrpl_b200.parallel import Comm
 comm = Comm()
 ini, t = bench.workload_inputs()
-rng = np.random.default_rng(1234)
-vals, uncs = bench.synth_measurement(lambda *a, **k: tme.eval_trial_moves(*a, cache=None, **k), ini, t, rng)
+vals, uncs = bench.workload_measurement()
 names = bench.NAMES
 param_info = {"names": list(names), "active": {n: int(n not in ("n0", "eps", "Tm", "m")) for n in names},
               "unit_conversions": dict(zip(names, bench.UNITS)), "do_log": {n: 1 for n in names},

@@ -7,8 +7,7 @@ import bench
 from metrotrpl_b200 import trial_move_evaluation as tme
 
 ini, t = bench.workload_inputs()
-rng = np.random.default_rng(1234)
-vals, uncs = bench.synth_measurement(lambda *a, **k: tme.eval_trial_moves(*a, cache=None, **k), ini, t, rng)
+vals, uncs = bench.workload_measurement()
 sf = bench.make_shared_fields(ini, t, vals, uncs)
 states = bench.draw_states(4096, seed=20261018)
 res = tme.eval_trial_moves(states, np.ones((4096, 3)), {"TRPL": 1.0}, sf)

@@ -20,7 +20,6 @@ sys.path.insert(0, ROOT)
 import bench  # noqa: E402
 from metrotrpl_b200 import dense_sampling as ds  # noqa: E402
 from metrotrpl_b200.parallel import Comm  # noqa: E402
-from metrotrpl_b200 import trial_move_evaluation as tme  # noqa: E402
 
 
 def main():
@@ -30,10 +29,8 @@ def main():
     args = ap.parse_args()
     comm = Comm()
     ini, t = bench.workload_inputs()
-    rng = np.random.default_rng(1234)
     os.environ["TRPL_USE_LOCAL_RANK"] = "1"
-    vals, uncs = bench.synth_measurement(
-        lambda *a, **k: tme.eval_trial_moves(*a, cache=tme.PathCache(a[3], device=comm.local_rank), **k), ini, t, rng)
+    vals, uncs = bench.workload_measurement()
     names = bench.NAMES
     param_info = {"names": list(names), "active": {n: int(n not in ("n0", "eps", "Tm", "m")) for n in names},
                   "unit_conversions": dict(zip(names, bench.UNITS)), "do_log": {n: 1 for n in names},
