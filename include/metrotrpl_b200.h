@@ -62,7 +62,7 @@ enum trpl_opt_flags { TRPL_OPT_FORCE_MIN_Y = 1, TRPL_OPT_NO_LIKELIHOOD = 2, TRPL
                                                     (csrc/extrapolation.h) instead of RODAS4; together with
                                                     TRPL_OPT_CTA_PER_TRAJ its six columns run in parallel on
                                                     the four warps of a CTA: a quarter of the latency per
-                                                    trajectory; 'std' model, nx = 128 only */ };
+                                                    trajectory; 'std' and 'traps' models, nx = 128 only */ };
 
 /* one measurement (sim_info["lengths"/"nx"/"meas_types"][i] + its slice of the data arrays) */
 typedef struct trpl_meas_desc {

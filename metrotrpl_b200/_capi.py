@@ -54,6 +54,14 @@ class SolverOpts(C.Structure):
                 ("max_steps", C.c_int32), ("flags", C.c_int32)]
 
 
+def check_extrapolation_problem(model, nx) -> None:
+    """Raise ValueError unless the problem can run on the low-latency extrapolation integrator
+    (OPT_EXTRAPOLATION, csrc/extrapolation.h): the 'std' or 'traps' model with nx = 128 on every
+    measurement.  model: name as in MODEL_IDS; nx: nodes of each measurement."""
+    if model not in ("std", "traps") or any(int(n) != 128 for n in nx):
+        raise ValueError("kernel='seulex' needs the 'std' or 'traps' model with nx = 128 on every measurement")
+
+
 def effective_tolerances(RTOL=None, ATOL=None):
     """Map the reference's (RTOL, ATOL) arguments onto the Rosenbrock controller."""
     rtol = DEFAULT_RTOL if RTOL is None else float(RTOL)

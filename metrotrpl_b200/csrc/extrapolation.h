@@ -351,19 +351,32 @@ TRPL_FN void run_trajectory_seulex(const TrajIn& in, const SolverOpts& opt, Traj
   out.status = status | em.status; out.n_acc = n_acc; out.n_rej = n_rej;
 }
 
+// Exchange area of the cooperative driver, behind the four warps' slices of shared memory: the
+// column increments as double2 (N, Q) [column][node][lane] and, for traps, their T components as
+// double [column][node][lane] behind those.  'std' keeps two such buffers, alternating by step
+// parity, and needs ONE __syncthreads per step.  Traps keeps one and adds a second __syncthreads once
+// every warp has read it: at 4 nodes per lane that is 18 432 B instead of 36 864, the CTA with its four
+// 23 040 B slices is 110.6 KB, and two CTAs still share an SM (2 x 129 KB would not fit its 228 KB).
+template <int NPL, int MODEL>
+struct SeulexXch {
+  static constexpr int PER_BUF = Seulex::K * NPL * 32;       // entries of each component array
+  static constexpr int BUFS = (MODEL == MODEL_TRAPS) ? 1 : 2;
+  static constexpr int BYTES = BUFS * PER_BUF * ((MODEL == MODEL_TRAPS) ? 16 + 8 : 16);
+};
+
 #if defined(__CUDACC__) && !defined(TRPL_HOST_EMU)
 // ---- driver 2: four warps of a CTA, columns in parallel ----------------------------------------
-// xch: 2 x (6 columns x NPL pairs) x 32 lanes of double2, double buffered by step parity; s_flag: one
-// int of shared memory for the rare step-log flush.  Every warp holds the full state (lane l owns the
-// same nodes in all four), computes its own columns, and after ONE __syncthreads per step combines
-// all six increments in the fixed order of the one-warp driver - identical bits, identical decisions.
+// xch: SeulexXch<NPL, MODEL>; s_flag: one int of shared memory for the rare step-log flush.  Every
+// warp holds the full state (lane l owns the same nodes in all four), computes its own columns, and
+// after a __syncthreads combines all six increments in the fixed order of the one-warp driver -
+// identical bits, identical decisions.
 template <int NPL, int MODEL, bool FULL>
 __device__ __forceinline__ void run_trajectory_seulex_cta(const TrajIn& in, const SolverOpts& opt, TrajMem& mem,
                                                           double2* xch, int* s_flag, int warp, TrajOut& out,
                                                           TrajMid& mid) {
   typedef Slots<NPL, MODEL> SL;
   typedef Vec<NPL, MODEL> V;
-  static_assert(MODEL == MODEL_STD, "the cooperative driver exchanges (N, Q) pairs only");
+  typedef SeulexXch<NPL, MODEL> XC;
   LaneMem& sm = mem.sm;
   const MeasDesc& md = *in.md;
   const int L = md.nx;
@@ -382,7 +395,7 @@ __device__ __forceinline__ void run_trajectory_seulex_cta(const TrajIn& in, cons
     ex_floor = EXCESS_RANGE * uni(warp_max(dn_max));
   }
   const double tend = in.times[md.n_t - 1];
-  const double inv_n = 1.0 / (2.0 * L);
+  const double inv_n = 1.0 / ((MODEL == MODEL_TRAPS) ? 3.0 * L : 2.0 * L);   // the one-warp driver's value
   const double h_min = 1e-14 * fmax(tend, 1e-300);
   double t = 0.0, h = 0.0, h_new = 0.0, h_cap = 0.0, val0 = 0.0, dval0 = 0.0, val_floor = 0.0;
   int status = ST_OK, n_acc = 0, n_rej = 0, nh = 0, buf = 0;
@@ -390,7 +403,8 @@ __device__ __forceinline__ void run_trajectory_seulex_cta(const TrajIn& in, cons
   Emitter em;
   emitter_init(em);
   typename PmChoice<SL>::type pf = PmChoice<SL>::make(mem);
-  constexpr int PER_BUF = Seulex::K * NPL * 32;        // double2 entries per buffer
+  constexpr int PER_BUF = XC::PER_BUF;
+  double* const xt = reinterpret_cast<double*>(xch + PER_BUF);      // traps: the T components
 
   while (!done) {
     {
@@ -434,7 +448,10 @@ __device__ __forceinline__ void run_trajectory_seulex_cta(const TrajIn& in, cons
       for (int ci = Seulex::group_first(warp); ci < Seulex::group_first(warp + 1); ++ci) {
         V d;
         seulex_column<NPL, MODEL>(Seulex::order(ci), ih, m, u, mem, pf, d);
-        TRPL_UNROLL for (int i = 0; i < NPL; ++i) xb[(ci * NPL + i) * 32 + lane] = make_double2(d.n[i], d.q[i]);
+        TRPL_UNROLL for (int i = 0; i < NPL; ++i) {
+          xb[(ci * NPL + i) * 32 + lane] = make_double2(d.n[i], d.q[i]);
+          if (MODEL == MODEL_TRAPS) xt[(ci * NPL + i) * 32 + lane] = d.t[i];
+        }
       }
       __syncthreads();
       V du, de, de5;
@@ -447,13 +464,15 @@ __device__ __forceinline__ void run_trajectory_seulex_cta(const TrajIn& in, cons
         TRPL_UNROLL for (int i = 0; i < NPL; ++i) {
           const double2 v = xb[(ci * NPL + i) * 32 + lane];
           d.n[i] = v.x; d.q[i] = v.y;
+          if (MODEL == MODEL_TRAPS) d.t[i] = xt[(ci * NPL + i) * 32 + lane];
         }
-        d.t[0] = 0.0;
+        if (MODEL != MODEL_TRAPS) d.t[0] = 0.0;
         vec_axpy<NPL, MODEL>(Seulex::A(j), d, du);
         vec_axpy<NPL, MODEL>(Seulex::B(j), d, de);
         vec_axpy<NPL, MODEL>(Seulex::B5(j), d, de5);
       }
-      buf ^= 1;
+      if (XC::BUFS == 1) __syncthreads();      // one buffer: read by every warp before the next columns write it
+      else buf ^= 1;
       V us;
       vec_add<NPL, MODEL>(u, du, us);
       bool nonfinite, nonfinite5;

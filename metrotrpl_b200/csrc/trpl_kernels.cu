@@ -128,7 +128,8 @@ __global__ void __launch_bounds__(32 * WARPS_PER_CTA, CTAS_PER_SM) trpl_seulex_k
 // The same integrator with the six columns of every step spread over the four warps of the CTA:
 // ONE trajectory per CTA, a quarter of the sequential depth.  Each warp keeps the full state and its
 // own factorisation storage (its slices of tensor and shared memory, as in trpl_forward_kernel); the
-// increments of the columns cross warps through a double-buffered exchange area behind the slices.
+// increments of the columns cross warps through an exchange area behind the slices (SeulexXch:
+// double-buffered for 'std', single-buffered for traps).
 template <int NPL, int MODEL, bool FULL>
 __global__ void __launch_bounds__(32 * WARPS_PER_CTA, CTAS_PER_SM) trpl_seulex_cta_kernel(const KernelArgs a) {
   typedef Slots<NPL, MODEL> SL;
@@ -412,15 +413,15 @@ int launch_cta(trpl_handle* h, KernelArgs a) {
 }
 
 // TRPL_OPT_EXTRAPOLATION: the order-6 extrapolation integrator, one warp per trajectory or (with
-// TRPL_OPT_CTA_PER_TRAJ) one CTA per trajectory.  'std' model, every measurement on 128 nodes.
-int launch_seulex(trpl_handle* h, KernelArgs a, bool cooperative) {
-  typedef Slots<4, MODEL_STD> SL;
-  if (h->model != TRPL_MODEL_STD || !h->all_full || h->max_nx != 128)
-    return fail("TRPL_OPT_EXTRAPOLATION: this integrator is built for the 'std' model with nx = 128 on every measurement");
+// TRPL_OPT_CTA_PER_TRAJ) one CTA per trajectory.  'std' or 'traps' model, every measurement on 128
+// nodes.
+template <int MODEL>
+int launch_seulex_model(trpl_handle* h, KernelArgs a, bool cooperative) {
+  typedef Slots<4, MODEL> SL;
   const int wpc = WARPS_PER_CTA;
-  const size_t xch_bytes = cooperative ? (size_t)2 * Seulex::K * 4 * 32 * sizeof(double2) : 0;
+  const size_t xch_bytes = cooperative ? (size_t)SeulexXch<4, MODEL>::BYTES : 0;
   const size_t smem = (size_t)wpc * SL::BYTES + xch_bytes;
-  auto kern = cooperative ? trpl_seulex_cta_kernel<4, MODEL_STD, true> : trpl_seulex_kernel<4, MODEL_STD, true>;
+  auto kern = cooperative ? trpl_seulex_cta_kernel<4, MODEL, true> : trpl_seulex_kernel<4, MODEL, true>;
   CU(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
   CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const int by_smem = (int)((size_t)h->prop.sharedMemPerMultiprocessor / (smem + 1024 + 16));
@@ -431,8 +432,8 @@ int launch_seulex(trpl_handle* h, KernelArgs a, bool cooperative) {
   int grid = std::min(h->prop.multiProcessorCount * per_sm, (a.n_traj + slots - 1) / slots);
   if (grid < 1) grid = 1;
   if (getenv("TRPL_DEBUG"))
-    fprintf(stderr, "[trpl] launch extrapolation (%s): %zu B smem/CTA, %d CTAs/SM, grid %d\n",
-            cooperative ? "one CTA per trajectory" : "one warp per trajectory", smem, per_sm, grid);
+    fprintf(stderr, "[trpl] launch extrapolation (%s), model=%d: %zu B smem/CTA, %d CTAs/SM, grid %d\n",
+            cooperative ? "one CTA per trajectory" : "one warp per trajectory", MODEL, smem, per_sm, grid);
   if (a.scratch) {
     CU(h->d_scratch.reserve((size_t)grid * slots * a.scratch_stride));
     a.scratch = h->d_scratch.p;
@@ -447,6 +448,17 @@ int launch_seulex(trpl_handle* h, KernelArgs a, bool cooperative) {
   h->launches += 1;
   CU(cudaEventRecord(h->ev1, h->stream));
   return 0;
+}
+
+int launch_seulex(trpl_handle* h, const KernelArgs& a, bool cooperative) {
+  if (!h->all_full || h->max_nx != 128)
+    return fail("TRPL_OPT_EXTRAPOLATION: this integrator is built for the 'std' and 'traps' models with nx = 128 on every measurement");
+  if (h->model == TRPL_MODEL_STD) return launch_seulex_model<MODEL_STD>(h, a, cooperative);
+#ifdef TRPL_DEV_HEADLINE_ONLY
+  return fail("this developer build only holds the 'std' model");
+#else
+  return launch_seulex_model<MODEL_TRAPS>(h, a, cooperative);
+#endif
 }
 
 template <int MODEL>

@@ -64,7 +64,9 @@ class CudaEvaluator:
         self.ladder = np.ascontiguousarray(shared_fields["_T"], dtype=np.float64)
         self.flags = self.cache.flags | _capi.OPT_LADDER
         sim = shared_fields["_sim_info"]
-        eligible = shared_fields.get("model", "std") == "std" and all(int(nx) == 128 for nx in sim["nx"])
+        model = shared_fields.get("model", "std")
+        # RODAS4 on a CTA (kernel="cta") exists for the 'std' model on 128 nodes only
+        eligible = model == "std" and all(int(nx) == 128 for nx in sim["nx"])
         n_global = int(shared_fields.get("_n_chains", 1)) * self.cache.n_meas
         if kernel not in ("auto", "warp", "cta", "seulex"):
             raise ValueError(f"unknown kernel {kernel!r}")
@@ -74,8 +76,7 @@ class CudaEvaluator:
             # iteration fits the GPU in one wave (<= ~300 trajectories per GPU), lower throughput
             # beyond.  A different integrator: results agree with RODAS4's to integration accuracy
             # (log-likelihoods to 2e-7), not bit for bit, so it is never chosen automatically.
-            if not eligible:
-                raise ValueError("kernel='seulex' needs the 'std' model with nx = 128 on every measurement")
+            _capi.check_extrapolation_problem(model, sim["nx"])
             self.flags |= _capi.OPT_EXTRAPOLATION | _capi.OPT_CTA_PER_TRAJ
         elif kernel == "cta" or (kernel == "auto" and eligible and n_global <= CTA_KERNEL_MAX_TRAJ):
             self.flags |= _capi.OPT_CTA_PER_TRAJ

@@ -43,7 +43,7 @@ class PathCache:
         kernel: "warp" (RODAS4, one trajectory per warp: throughput) or "seulex" (order-6
         extrapolation, one trajectory per CTA, csrc/extrapolation.h: half the latency for batches of
         a few hundred trajectories - single states, Nelder-Mead simplices, tempering ladders; 'std'
-        model with nx = 128 only)."""
+        or 'traps' model with nx = 128 only)."""
         sf = shared_fields
         if any(m == "pa" for m in sf["_sim_info"]["meas_types"]):
             raise NotImplementedError("'pa' toy measurements are not simulations; not on the CUDA path")
@@ -84,8 +84,7 @@ class PathCache:
         self.s_idx = group_index(sf.get("scale_factor", None), "_s")
         self.flags = _capi.OPT_FORCE_MIN_Y if sf.get("force_min_y", False) else 0
         if kernel == "seulex":
-            if sf.get("model", "std") != "std" or any(int(nx) != 128 for nx in sf["_sim_info"]["nx"]):
-                raise ValueError("kernel='seulex' needs the 'std' model with nx = 128 on every measurement")
+            _capi.check_extrapolation_problem(sf.get("model", "std"), sf["_sim_info"]["nx"])
             self.flags |= _capi.OPT_EXTRAPOLATION | _capi.OPT_CTA_PER_TRAJ
         elif kernel != "warp":
             raise ValueError(f"unknown kernel {kernel!r}")
