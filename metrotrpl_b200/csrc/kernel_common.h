@@ -1,12 +1,24 @@
-// kernel_common.h - what the two translation units of the library share: the launch arguments, the
-// per-trajectory set-up / result write-back and the tensor-memory slice of a warp.
+// kernel_common.h - what the translation units of the library share: the launch arguments and plan,
+// the work queue, the per-trajectory set-up / result write-back and the tensor-memory slice of a warp.
 //   trpl_kernels.cu   one warp per trajectory (simt.h with TRPL_TEAM == 1), the C ABI
 //   team_kernels.cu   a team of two warps per trajectory (TRPL_TEAM == 2): the grids of 129..256 nodes
-// Included inside each unit after trajectory.h; everything here has internal linkage.
+//   team4_kernels.cu  a team of four warps per trajectory (TRPL_TEAM == 4): the grids of 257..512 nodes
+// Included inside each unit after trajectory.h; everything here except LaunchPlan has internal linkage.
 #pragma once
 #include <cuda_runtime.h>
 #include "../../include/metrotrpl_b200.h"
 #include "trajectory.h"
+
+// How one launch of a persistent trajectory kernel is shaped (run_plan in trpl_kernels.cu runs it).
+// Global scope: the team units fill it for their kernels, so every unit sees one layout.
+struct LaunchPlan {
+  const void* kernel;            // first pass
+  const void* explicit_kernel;   // second pass over the trajectories the first deferred, or null
+  int block;                     // threads per CTA
+  size_t smem;                   // dynamic shared memory per CTA (0: static only)
+  int tm_cols;                   // tensor-memory columns per CTA (0: none)
+  int traj_per_cta;              // concurrent trajectories per CTA = step-log / scratch slices per CTA
+};
 
 namespace {
 
@@ -32,7 +44,7 @@ struct KernelArgs {
   int* nsteps;               // [n_traj][2]
   double* curves;            // [n_sets][n_times_total] or null
   const double* irf_mom;     // [rows][3] or null
-  double* scratch;           // per-warp slices: resampled | convolved | trimmed
+  double* scratch;           // per-slot slices: resampled | convolved | trimmed
   size_t scratch_stride, off_hk, off_trim, off_r2, off_u2;
   const double* ladder_T;
   double* ladder_out;        // [n_traj][n_ladder]
@@ -40,15 +52,41 @@ struct KernelArgs {
   int* counter;              // work queue head
   const int* meas_order;     // [n_meas] measurement indices, most expensive first
   const int* queue;          // [n_traj] explicit queue order (trpl_set_queue_order) or null
-  double* hist;              // per-warp step histories, 3 * HIST_CAP doubles each
+  double* hist;              // per-slot step histories, 3 * HIST_CAP doubles each
   int* defer_list;           // trajectories handed to the explicit path
   int* defer_count;
-  int n_traj, n_meas, n_times_total, warps_per_cta;
+  int n_traj, n_meas, n_times_total;
+  int slots_per_cta;         // trajectories a CTA runs at once (warps, teams or 1): step-log / scratch slices
   SolverOpts opt;
 };
 
+// Queue position -> trajectory index (results are indexed [set][meas]).  Without an explicit order
+// the queue is measurement-major with the (statically) most expensive curves first, so that the
+// tail of the launch is made of the cheapest trajectories.
+__device__ __forceinline__ int queue_traj(const KernelArgs& a, int q) {
+  if (a.queue) return a.queue[q];
+  const int n_sets_q = a.n_traj / a.n_meas;
+  const int qm = q / n_sets_q;
+  return (q - qm * n_sets_q) * a.n_meas + a.meas_order[qm];
+}
+
+// next queue position of a warp: lane 0 claims it, every lane receives it
+__device__ __forceinline__ int warp_claim(int* counter, int lane) {
+  int q = 0;
+  if (lane == 0) q = atomicAdd(counter, 1);
+  return __shfl_sync(0xffffffffu, q, 0);
+}
+
+// next queue position of a CTA: thread 0 claims it into the __shared__ `slot`, every thread reads it
+__device__ __forceinline__ int cta_claim(int* counter, int* slot) {
+  __syncthreads();
+  if (threadIdx.x == 0) *slot = atomicAdd(counter, 1);
+  __syncthreads();
+  return *slot;
+}
+
 __device__ __forceinline__ void setup_traj(const KernelArgs& a, int traj, int warp, TrajIn& in) {
-  in.hist = a.hist + (size_t)(blockIdx.x * a.warps_per_cta + warp) * (3 * HIST_CAP);
+  in.hist = a.hist + (size_t)(blockIdx.x * a.slots_per_cta + warp) * (3 * HIST_CAP);
   const int set = traj / a.n_meas;
   const int mi = traj - set * a.n_meas;
   const MeasDesc* md = a.meas + mi;
@@ -79,7 +117,7 @@ __device__ __forceinline__ void finish_traj(const KernelArgs& a, int traj, int w
   tl.irf.nk = conv ? md->irf_nk : 0;
   tl.irf.dt = md->irf_dt;
   tl.irf.mom = a.irf_mom ? a.irf_mom + 3 * (size_t)md->irf_off : nullptr;
-  double* ws = a.scratch ? a.scratch + (size_t)(blockIdx.x * a.warps_per_cta + warp) * a.scratch_stride : nullptr;
+  double* ws = a.scratch ? a.scratch + (size_t)(blockIdx.x * a.slots_per_cta + warp) * a.scratch_stride : nullptr;
   tl.irf.ry = ws; tl.irf.hk = ws ? ws + a.off_hk : nullptr; tl.irf.trim = ws ? ws + a.off_trim : nullptr;
   tl.r2_scratch = (ws && ladder) ? ws + a.off_r2 : nullptr;
   tl.u2_scratch = (ws && ladder) ? ws + a.off_u2 : nullptr;

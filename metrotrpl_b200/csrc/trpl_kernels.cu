@@ -41,19 +41,9 @@ __global__ void __launch_bounds__(32 * WARPS_PER_CTA, CTAS_PER_SM) trpl_forward_
   TrajMem mem{LaneMem{smem + warp * (SL::COUNT * 32)}, tmem_acquire<SL>(warp)};   // COUNT pairs of 16 B per lane
   const bool allow_defer = a.defer_list != nullptr;
   for (;;) {
-    int traj = 0;
-    if (lane == 0) traj = atomicAdd(a.counter, 1);
-    traj = __shfl_sync(0xffffffffu, traj, 0);
-    if (traj >= a.n_traj) break;
-    // queue order is measurement-major with the (statically) most expensive curves first, so that
-    // the tail of the launch is made of the cheapest trajectories; results are indexed [set][meas]
-    if (a.queue) {
-      traj = a.queue[traj];
-    } else {
-      const int n_sets_q = a.n_traj / a.n_meas;
-      const int qm = traj / n_sets_q;
-      traj = (traj - qm * n_sets_q) * a.n_meas + a.meas_order[qm];
-    }
+    const int q = warp_claim(a.counter, lane);
+    if (q >= a.n_traj) break;
+    const int traj = queue_traj(a, q);
     TrajIn in;
     setup_traj(a, traj, warp, in);
     TrajOut out;
@@ -77,9 +67,7 @@ __global__ void __launch_bounds__(32 * WARPS_PER_CTA, CTAS_PER_SM) trpl_explicit
   TrajMem mem{LaneMem{smem + warp * (SL::COUNT * 32)}, tmem_acquire<SL>(warp)};
   const int n = *a.defer_count;
   for (;;) {
-    int q = 0;
-    if (lane == 0) q = atomicAdd(a.counter + 1, 1);
-    q = __shfl_sync(0xffffffffu, q, 0);
+    const int q = warp_claim(a.counter + 1, lane);
     if (q >= n) break;
     const int traj = a.defer_list[q];
     TrajIn in;
@@ -104,17 +92,9 @@ __global__ void __launch_bounds__(32 * WARPS_PER_CTA, CTAS_PER_SM) trpl_seulex_k
   const int lane = threadIdx.x & 31;
   TrajMem mem{LaneMem{smem + warp * (SL::COUNT * 32)}, tmem_acquire<SL>(warp)};
   for (;;) {
-    int traj = 0;
-    if (lane == 0) traj = atomicAdd(a.counter, 1);
-    traj = __shfl_sync(0xffffffffu, traj, 0);
-    if (traj >= a.n_traj) break;
-    if (a.queue) {
-      traj = a.queue[traj];
-    } else {
-      const int n_sets_q = a.n_traj / a.n_meas;
-      const int qm = traj / n_sets_q;
-      traj = (traj - qm * n_sets_q) * a.n_meas + a.meas_order[qm];
-    }
+    const int q = warp_claim(a.counter, lane);
+    if (q >= a.n_traj) break;
+    const int traj = queue_traj(a, q);
     TrajIn in;
     setup_traj(a, traj, warp, in);
     TrajOut out;
@@ -139,20 +119,11 @@ __global__ void __launch_bounds__(32 * WARPS_PER_CTA, CTAS_PER_SM) trpl_seulex_c
   TrajMem mem{LaneMem{smem + warp * (SL::COUNT * 32)}, tmem_acquire<SL>(warp)};
   double2* xch = smem + WARPS_PER_CTA * (SL::COUNT * 32);
   for (;;) {
-    __syncthreads();
-    if (threadIdx.x == 0) s_traj = atomicAdd(a.counter, 1);
-    __syncthreads();
-    int traj = s_traj;
-    if (traj >= a.n_traj) break;
-    if (a.queue) {
-      traj = a.queue[traj];
-    } else {
-      const int n_sets_q = a.n_traj / a.n_meas;
-      const int qm = traj / n_sets_q;
-      traj = (traj - qm * n_sets_q) * a.n_meas + a.meas_order[qm];
-    }
+    const int q = cta_claim(a.counter, &s_traj);
+    if (q >= a.n_traj) break;
+    const int traj = queue_traj(a, q);
     TrajIn in;
-    setup_traj(a, traj, 0, in);               // warps_per_cta == 1: one step log / scratch slice per CTA
+    setup_traj(a, traj, 0, in);               // slots_per_cta == 1: one step log / scratch slice per CTA
     TrajOut out;
     TrajMid mid;
     run_trajectory_seulex_cta<NPL, MODEL, FULL>(in, a.opt, mem, xch, &s_flag, warp, out, mid);
@@ -166,18 +137,9 @@ __global__ void __launch_bounds__(32 * WARPS_PER_CTA, CTAS_PER_SM) trpl_seulex_c
 __global__ void __launch_bounds__(cta::NX, 2) trpl_cta_kernel(const KernelArgs a) {
   __shared__ cta::Smem s;
   for (;;) {
-    __syncthreads();
-    if (threadIdx.x == 0) s.traj = atomicAdd(a.counter, 1);
-    __syncthreads();
-    int traj = s.traj;
-    if (traj >= a.n_traj) break;
-    if (a.queue) {
-      traj = a.queue[traj];
-    } else {
-      const int n_sets_q = a.n_traj / a.n_meas;
-      const int qm = traj / n_sets_q;
-      traj = (traj - qm * n_sets_q) * a.n_meas + a.meas_order[qm];
-    }
+    const int q = cta_claim(a.counter, &s.traj);
+    if (q >= a.n_traj) break;
+    const int traj = queue_traj(a, q);
     TrajIn in;
     setup_traj(a, traj, 0, in);
     TrajOut out;
@@ -266,188 +228,110 @@ struct trpl_handle {
 
 namespace {
 
-template <int NPL, int MODEL, bool FULL>
-int launch(trpl_handle* h, KernelArgs a) {
-  // warps per CTA: at most four (one per tensor-memory lane quarter), fewer if their shared-memory
-  // slices do not fit the 227 KB of one CTA (the larger grids)
-  typedef Slots<NPL, MODEL> SL;
-  const size_t per_warp = SL::BYTES;
-  int wpc = WARPS_PER_CTA;
-  while (wpc > 1 && (size_t)wpc * per_warp > (size_t)h->prop.sharedMemPerBlockOptin) --wpc;
-  if ((size_t)wpc * per_warp > (size_t)h->prop.sharedMemPerBlockOptin)
-    return fail("trajectory state does not fit in shared memory");
-  size_t smem = (size_t)wpc * per_warp;
-  a.warps_per_cta = wpc;
-  auto kern = trpl_forward_kernel<NPL, MODEL, FULL>;
-  // the occupancy calculator assumes the function's current carve-out: ask for the largest one
-  // first, or a small shared-memory request is judged against a small default carve-out
-  CU(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-  CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+// Runs one launch plan: residency, grid, per-slot buffers, then the kernel and (unless
+// TRPL_OPT_NO_EXPLICIT) the explicit second pass over the trajectories it deferred.
+int run_plan(trpl_handle* h, KernelArgs a, const LaunchPlan& p, const char* what) {
+  if (p.smem > (size_t)h->prop.sharedMemPerBlockOptin) return fail("trajectory state does not fit in shared memory");
+  const bool two_pass = p.explicit_kernel && !(a.opt.flags & OPT_NO_EXPLICIT);
+  if (p.smem > 0) {
+    // the occupancy calculator assumes the function's current carve-out: ask for the largest one
+    // first, or a small shared-memory request is judged against a small default carve-out
+    for (const void* k : {p.kernel, p.explicit_kernel}) {
+      if (!k) continue;
+      CU(cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+      CU(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem));
+    }
+  }
   int per_sm = 0;
-  CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, 32 * wpc, smem));
-  if (per_sm < 1) return fail("trajectory kernel does not fit on an SM");
+  CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, p.kernel, p.block, p.smem));
   // CTAs resident on an SM share its 512 tensor-memory columns (a CTA beyond that would sit in
   // tcgen05.alloc until another one exits).  The occupancy calculator answers 1 for any kernel
   // that allocates tensor memory, so residency is computed here: registers and shared memory
   // (launch bounds), capped by the tensor-memory columns.
-  if (SL::TM_COUNT > 0) {
-    const int by_smem = (int)((size_t)h->prop.sharedMemPerMultiprocessor / (smem + 1024 + 16));
-    per_sm = std::min(std::min(CTAS_PER_SM * WARPS_PER_CTA / wpc, by_smem), 512 / TmCta<SL>::COLS);
-    if (per_sm < 1) return fail("trajectory kernel does not fit on an SM");
+  if (per_sm >= 1 && p.tm_cols > 0) {
+    const int by_smem = (int)((size_t)h->prop.sharedMemPerMultiprocessor / (p.smem + 1024 + 16));
+    per_sm = std::min({CTAS_PER_SM * WARPS_PER_CTA / (p.block / 32), by_smem, 512 / p.tm_cols});
   }
-  CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  const int warps_needed = a.n_traj;
-  int grid = h->prop.multiProcessorCount * per_sm;
-  const int ctas_needed = (warps_needed + wpc - 1) / wpc;
-  if (grid > ctas_needed) grid = ctas_needed;
-  if (grid < 1) grid = 1;
-  if (getenv("TRPL_DEBUG"))
-    fprintf(stderr, "[trpl] launch NPL=%d model=%d: %d warps/CTA, %zu B smem/CTA, %d TMEM columns/CTA, %d CTAs/SM, grid %d\n",
-            NPL, MODEL, wpc, smem, SL::TM_COUNT > 0 ? TmCta<SL>::COLS : 0, per_sm, grid);
-  if (a.scratch) {
-    CU(h->d_scratch.reserve((size_t)grid * wpc * a.scratch_stride));
+  if (per_sm < 1) return fail(std::string(what) + " does not fit on an SM");
+  const int grid = std::max(1, std::min(h->prop.multiProcessorCount * per_sm,
+                                        (a.n_traj + p.traj_per_cta - 1) / p.traj_per_cta));
+  if (getenv("TRPL_DEBUG")) {
+    cudaFuncAttributes fa;
+    CU(cudaFuncGetAttributes(&fa, p.kernel));
+    fprintf(stderr, "[trpl] launch %s, model=%d: %d threads/CTA, %d trajectories/CTA, %zu B dynamic + %zu B static smem/CTA, "
+            "%d TMEM columns/CTA, %d CTAs/SM, grid %d\n", what, h->model, p.block, p.traj_per_cta, p.smem,
+            fa.sharedSizeBytes, p.tm_cols, per_sm, grid);
+  }
+  a.slots_per_cta = p.traj_per_cta;
+  if (a.scratch_stride > 0) {
+    CU(h->d_scratch.reserve((size_t)grid * p.traj_per_cta * a.scratch_stride));
     a.scratch = h->d_scratch.p;
   }
-  CU(h->d_hist.reserve((size_t)grid * wpc * 3 * HIST_CAP));
+  CU(h->d_hist.reserve((size_t)grid * p.traj_per_cta * 3 * HIST_CAP));
   a.hist = h->d_hist.p;
   CU(cudaMemsetAsync(h->d_counter.p, 0, 4 * sizeof(int), h->stream));
   a.defer_list = nullptr; a.defer_count = h->d_counter.p + 2;
-  if (!(a.opt.flags & OPT_NO_EXPLICIT)) {
+  if (two_pass) {
     CU(h->d_defer.reserve(a.n_traj));
     a.defer_list = h->d_defer.p;
   }
+  void* args[] = {&a};
   CU(cudaEventRecord(h->ev0, h->stream));
-  kern<<<grid, 32 * wpc, smem, h->stream>>>(a);
-  CU(cudaGetLastError());
-  h->launches += 1;
-  if (a.defer_list) {
-    auto kern2 = trpl_explicit_kernel<NPL, MODEL, FULL>;
-    CU(cudaFuncSetAttribute(kern2, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    CU(cudaFuncSetAttribute(kern2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kern2<<<grid, 32 * wpc, smem, h->stream>>>(a);
-    CU(cudaGetLastError());
+  for (const void* k : {p.kernel, two_pass ? p.explicit_kernel : nullptr}) {
+    if (!k) continue;
+    CU(cudaLaunchKernel(k, grid, p.block, args, p.smem, h->stream));
     h->launches += 1;
   }
   CU(cudaEventRecord(h->ev1, h->stream));
   return 0;
+}
+
+// One warp per trajectory: at most four warps per CTA (one per tensor-memory lane quarter), fewer if
+// their shared-memory slices do not fit the 227 KB of one CTA (the larger grids).
+template <int NPL, int MODEL, bool FULL>
+int launch(trpl_handle* h, const KernelArgs& a) {
+  typedef Slots<NPL, MODEL> SL;
+  int wpc = WARPS_PER_CTA;
+  while (wpc > 1 && (size_t)wpc * SL::BYTES > (size_t)h->prop.sharedMemPerBlockOptin) --wpc;
+  const LaunchPlan p{(const void*)trpl_forward_kernel<NPL, MODEL, FULL>, (const void*)trpl_explicit_kernel<NPL, MODEL, FULL>,
+                     32 * wpc, (size_t)wpc * SL::BYTES, TmCta<SL>::COLS, wpc};
+  return run_plan(h, a, p, "trajectory kernel");
 }
 
 // Grids of 129..256 / 257..512 nodes: a team of two / four warps per trajectory, compiled in
 // team_kernels.cu / team4_kernels.cu against the team vocabularies of simt.h (4 nodes per lane on 64 /
 // 128 lanes).  Same queue, same arguments, same per-trajectory scratch as launch<>; a CTA of four
-// warps holds two trajectories, or one.
-extern "C" void trpl_team_plan(int model, size_t* smem, int* tm_cols, int* teams_per_cta);
-extern "C" int trpl_team_run(int model, int full, const void* args, size_t args_size, int grid, size_t smem,
-                             void* stream, int explicit_pass);
-extern "C" void trpl_team4_plan(int model, size_t* smem, int* tm_cols, int* teams_per_cta);
-extern "C" int trpl_team4_run(int model, int full, const void* args, size_t args_size, int grid, size_t smem,
-                              void* stream, int explicit_pass);
+// warps holds two trajectories, or one.  Each unit hands out its plan and its sizeof(KernelArgs).
+extern "C" size_t trpl_team_plan(int model, int full, LaunchPlan* out);
+extern "C" size_t trpl_team4_plan(int model, int full, LaunchPlan* out);
 
-int launch_team(trpl_handle* h, KernelArgs a, int team_warps) {
-  size_t smem = 0;
-  int cols = 0, tpc = 1;
-  const auto plan = team_warps == 4 ? trpl_team4_plan : trpl_team_plan;
-  const auto run = team_warps == 4 ? trpl_team4_run : trpl_team_run;
-  plan(h->model, &smem, &cols, &tpc);
-  if (smem > (size_t)h->prop.sharedMemPerBlockOptin) return fail("trajectory state does not fit in shared memory");
-  const int by_smem = (int)((size_t)h->prop.sharedMemPerMultiprocessor / (smem + 1024 + 16));
-  int per_sm = std::min(CTAS_PER_SM, by_smem);
-  if (cols > 0) per_sm = std::min(per_sm, 512 / cols);
-  if (per_sm < 1) return fail("team kernel does not fit on an SM");
-  a.warps_per_cta = tpc;                      // step logs / scratch slices: one per team
-  int grid = std::min(h->prop.multiProcessorCount * per_sm, (a.n_traj + tpc - 1) / tpc);
-  if (grid < 1) grid = 1;
-  if (getenv("TRPL_DEBUG"))
-    fprintf(stderr, "[trpl] launch %d-warp teams, model=%d full=%d: %d teams/CTA, %zu B smem/CTA, %d TMEM columns/CTA, %d CTAs/SM, grid %d\n",
-            team_warps, h->model, (int)h->all_full, tpc, smem, cols, per_sm, grid);
-  if (a.scratch) {
-    CU(h->d_scratch.reserve((size_t)grid * tpc * a.scratch_stride));
-    a.scratch = h->d_scratch.p;
-  }
-  CU(h->d_hist.reserve((size_t)grid * tpc * 3 * HIST_CAP));
-  a.hist = h->d_hist.p;
-  CU(cudaMemsetAsync(h->d_counter.p, 0, 4 * sizeof(int), h->stream));
-  a.defer_list = nullptr; a.defer_count = h->d_counter.p + 2;
-  if (!(a.opt.flags & OPT_NO_EXPLICIT)) {
-    CU(h->d_defer.reserve(a.n_traj));
-    a.defer_list = h->d_defer.p;
-  }
+int launch_team(trpl_handle* h, const KernelArgs& a, int team_warps) {
+  LaunchPlan p;
   const int full = (h->all_full && h->max_nx == 128 * team_warps) ? 1 : 0;
-  CU(cudaEventRecord(h->ev0, h->stream));
-  CU((cudaError_t)run(h->model, full, &a, sizeof(a), grid, smem, h->stream, 0));
-  h->launches += 1;
-  if (a.defer_list) {
-    CU((cudaError_t)run(h->model, full, &a, sizeof(a), grid, smem, h->stream, 1));
-    h->launches += 1;
-  }
-  CU(cudaEventRecord(h->ev1, h->stream));
-  return 0;
+  if ((team_warps == 4 ? trpl_team4_plan : trpl_team_plan)(h->model, full, &p) != sizeof(KernelArgs))
+    return fail("the team kernel unit was built with another KernelArgs layout");
+  return run_plan(h, a, p, "team kernel");
 }
 
 // CTA-per-trajectory launch (TRPL_OPT_CTA_PER_TRAJ): 'std' model, every measurement on 128 nodes
-int launch_cta(trpl_handle* h, KernelArgs a) {
+int launch_cta(trpl_handle* h, const KernelArgs& a) {
   if (h->model != TRPL_MODEL_STD || !h->all_full || h->max_nx != cta::NX)
     return fail("TRPL_OPT_CTA_PER_TRAJ: this instantiation exists for the 'std' model with nx = 128 on every measurement");
-  a.warps_per_cta = 1;        // one step log / scratch slice per CTA (warp 0 runs the emission)
-  int per_sm = 0;
-  CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, trpl_cta_kernel, cta::NX, 0));
-  if (per_sm < 1) return fail("CTA-per-trajectory kernel does not fit on an SM");
-  int grid = std::min(h->prop.multiProcessorCount * per_sm, a.n_traj);
-  if (grid < 1) grid = 1;
-  if (getenv("TRPL_DEBUG"))
-    fprintf(stderr, "[trpl] launch CTA-per-trajectory: %d CTAs/SM, grid %d, %zu B smem/CTA\n", per_sm, grid, sizeof(cta::Smem));
-  if (a.scratch) {
-    CU(h->d_scratch.reserve((size_t)grid * a.scratch_stride));
-    a.scratch = h->d_scratch.p;
-  }
-  CU(h->d_hist.reserve((size_t)grid * 3 * HIST_CAP));
-  a.hist = h->d_hist.p;
-  CU(cudaMemsetAsync(h->d_counter.p, 0, 4 * sizeof(int), h->stream));
-  a.defer_list = nullptr; a.defer_count = h->d_counter.p + 2;
-  CU(cudaEventRecord(h->ev0, h->stream));
-  trpl_cta_kernel<<<grid, cta::NX, 0, h->stream>>>(a);
-  CU(cudaGetLastError());
-  h->launches += 1;
-  CU(cudaEventRecord(h->ev1, h->stream));
-  return 0;
+  // static shared memory only; one step log / scratch slice per CTA (warp 0 runs the emission)
+  return run_plan(h, a, LaunchPlan{(const void*)trpl_cta_kernel, nullptr, cta::NX, 0, 0, 1}, "CTA-per-trajectory kernel");
 }
 
 // TRPL_OPT_EXTRAPOLATION: the order-6 extrapolation integrator, one warp per trajectory or (with
 // TRPL_OPT_CTA_PER_TRAJ) one CTA per trajectory.  'std' or 'traps' model, every measurement on 128
 // nodes.
 template <int MODEL>
-int launch_seulex_model(trpl_handle* h, KernelArgs a, bool cooperative) {
+int launch_seulex_model(trpl_handle* h, const KernelArgs& a, bool cooperative) {
   typedef Slots<4, MODEL> SL;
-  const int wpc = WARPS_PER_CTA;
-  const size_t xch_bytes = cooperative ? (size_t)SeulexXch<4, MODEL>::BYTES : 0;
-  const size_t smem = (size_t)wpc * SL::BYTES + xch_bytes;
-  auto kern = cooperative ? trpl_seulex_cta_kernel<4, MODEL, true> : trpl_seulex_kernel<4, MODEL, true>;
-  CU(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-  CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  const int by_smem = (int)((size_t)h->prop.sharedMemPerMultiprocessor / (smem + 1024 + 16));
-  const int per_sm = std::min(std::min(CTAS_PER_SM, by_smem), 512 / TmCta<SL>::COLS);
-  if (per_sm < 1) return fail("extrapolation kernel does not fit on an SM");
-  a.warps_per_cta = cooperative ? 1 : wpc;
-  const int slots = cooperative ? 1 : wpc;                       // trajectories per CTA
-  int grid = std::min(h->prop.multiProcessorCount * per_sm, (a.n_traj + slots - 1) / slots);
-  if (grid < 1) grid = 1;
-  if (getenv("TRPL_DEBUG"))
-    fprintf(stderr, "[trpl] launch extrapolation (%s), model=%d: %zu B smem/CTA, %d CTAs/SM, grid %d\n",
-            cooperative ? "one CTA per trajectory" : "one warp per trajectory", MODEL, smem, per_sm, grid);
-  if (a.scratch) {
-    CU(h->d_scratch.reserve((size_t)grid * slots * a.scratch_stride));
-    a.scratch = h->d_scratch.p;
-  }
-  CU(h->d_hist.reserve((size_t)grid * slots * 3 * HIST_CAP));
-  a.hist = h->d_hist.p;
-  CU(cudaMemsetAsync(h->d_counter.p, 0, 4 * sizeof(int), h->stream));
-  a.defer_list = nullptr; a.defer_count = h->d_counter.p + 2;
-  CU(cudaEventRecord(h->ev0, h->stream));
-  kern<<<grid, 32 * wpc, smem, h->stream>>>(a);
-  CU(cudaGetLastError());
-  h->launches += 1;
-  CU(cudaEventRecord(h->ev1, h->stream));
-  return 0;
+  const LaunchPlan p{cooperative ? (const void*)trpl_seulex_cta_kernel<4, MODEL, true> : (const void*)trpl_seulex_kernel<4, MODEL, true>,
+                     nullptr, 32 * WARPS_PER_CTA,
+                     (size_t)WARPS_PER_CTA * SL::BYTES + (cooperative ? (size_t)SeulexXch<4, MODEL>::BYTES : 0),
+                     TmCta<SL>::COLS, cooperative ? 1 : WARPS_PER_CTA};
+  return run_plan(h, a, p, "extrapolation kernel");
 }
 
 int launch_seulex(trpl_handle* h, const KernelArgs& a, bool cooperative) {
@@ -780,8 +664,7 @@ int trpl_run_resident(trpl_handle* h, const trpl_solver_opts* opts, int32_t want
     a.off_trim = a.off_hk + ((n_hk + 3) & ~(size_t)3);
     a.off_r2 = a.off_trim + nt4;
     a.off_u2 = a.off_r2 + nt4;
-    a.scratch_stride = a.off_u2 + nt4;
-    a.scratch = reinterpret_cast<double*>(1);   // "wanted": sized and set in launch()
+    a.scratch_stride = a.off_u2 + nt4;        // run_plan sizes the slices and sets a.scratch
     if (conv) a.irf_mom = h->d_irf.p;
   }
   if (ladder) {

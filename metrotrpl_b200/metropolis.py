@@ -45,43 +45,24 @@ def roll_acceptance(rng, logratio):
     return rng.random() < np.exp(logratio)
 
 
-# A tempering iteration is as slow as its slowest trajectory.  The CTA-per-trajectory kernel
-# (csrc/cta_trajectory.h) was built for that case, but measured on B200 it has the SAME latency per
-# integrator step as the one-warp kernel (6.5 us: a step is a chain of ~50 dependent
-# exchange-and-reduce levels either way, tools/latency_probe.py, DESIGN.md section 5) at 0.3x the
-# throughput, so "auto" never picks it.  The choice is made from the GLOBAL number of trajectories
-# per iteration, never from this rank's share, so that a run gives the same chains on any number of
-# GPUs.
-CTA_KERNEL_MAX_TRAJ = 0
-
-
 class CudaEvaluator:
     """Likelihood of a batch of states at every ladder temperature, on this rank's GPU."""
 
     def __init__(self, shared_fields, device=None, kernel="auto"):
         from .trial_move_evaluation import PathCache
-        self.cache = PathCache(shared_fields, device=device)
-        self.ladder = np.ascontiguousarray(shared_fields["_T"], dtype=np.float64)
-        self.flags = self.cache.flags | _capi.OPT_LADDER
-        sim = shared_fields["_sim_info"]
-        model = shared_fields.get("model", "std")
-        # RODAS4 on a CTA (kernel="cta") exists for the 'std' model on 128 nodes only
-        eligible = model == "std" and all(int(nx) == 128 for nx in sim["nx"])
-        n_global = int(shared_fields.get("_n_chains", 1)) * self.cache.n_meas
         if kernel not in ("auto", "warp", "cta", "seulex"):
             raise ValueError(f"unknown kernel {kernel!r}")
-        if kernel == "seulex":
-            # order-6 extrapolation integrator, its columns in parallel on the four warps of a CTA
-            # (csrc/extrapolation.h): 1.4-2x lower latency per trajectory than RODAS4 while the whole
-            # iteration fits the GPU in one wave (<= ~300 trajectories per GPU), lower throughput
-            # beyond.  A different integrator: results agree with RODAS4's to integration accuracy
-            # (log-likelihoods to 2e-7), not bit for bit, so it is never chosen automatically.
-            _capi.check_extrapolation_problem(model, sim["nx"])
-            self.flags |= _capi.OPT_EXTRAPOLATION | _capi.OPT_CTA_PER_TRAJ
-        elif kernel == "cta" or (kernel == "auto" and eligible and n_global <= CTA_KERNEL_MAX_TRAJ):
-            self.flags |= _capi.OPT_CTA_PER_TRAJ
-        self.kernel = ("seulex" if self.flags & _capi.OPT_EXTRAPOLATION else
-                       "cta" if self.flags & _capi.OPT_CTA_PER_TRAJ else "warp")
+        # "auto" is RODAS4 with one trajectory per warp.  A tempering iteration is as slow as its
+        # slowest trajectory, but measured on B200, RODAS4 on a whole CTA ("cta",
+        # csrc/cta_trajectory.h) has the SAME latency per integrator step (6.5 us: a step is a chain
+        # of ~50 dependent exchange-and-reduce levels either way, tools/latency_probe.py, DESIGN.md
+        # section 5) at 0.3x the throughput.  "seulex" (csrc/extrapolation.h) is a different
+        # integrator: log-likelihoods agree with RODAS4's to 2e-7, not bit for bit, so it is never
+        # chosen automatically.
+        self.kernel = "warp" if kernel == "auto" else kernel
+        self.cache = PathCache(shared_fields, device=device, kernel=self.kernel)
+        self.ladder = np.ascontiguousarray(shared_fields["_T"], dtype=np.float64)
+        self.flags = self.cache.flags | _capi.OPT_LADDER
         self._cost = None       # integrator steps of the previous call's trajectories
         # trajectories this GPU holds at once (148 SMs x 2 CTAs x 4 warps, or x 1 per CTA): a batch
         # that fits starts all at once and the queue order (and the step counts it needs) is moot

@@ -40,10 +40,11 @@ class PathCache:
     def __init__(self, shared_fields, device=None, ctx=None, kernel="warp"):
         """ctx: a private _capi.Context (own stream and device buffers) instead of the process-wide
         one of `device`; two caches on two contexts let consecutive launches overlap.
-        kernel: "warp" (RODAS4, one trajectory per warp: throughput) or "seulex" (order-6
-        extrapolation, one trajectory per CTA, csrc/extrapolation.h: half the latency for batches of
-        a few hundred trajectories - single states, Nelder-Mead simplices, tempering ladders; 'std'
-        or 'traps' model with nx = 128 only)."""
+        kernel: "warp" (RODAS4, one trajectory per warp: throughput), "cta" (RODAS4 on a whole CTA,
+        csrc/cta_trajectory.h; 'std' model with nx = 128 only, refused at launch otherwise) or
+        "seulex" (order-6 extrapolation, one trajectory per CTA, csrc/extrapolation.h: half the
+        latency for batches of a few hundred trajectories - single states, Nelder-Mead simplices,
+        tempering ladders; 'std' or 'traps' model with nx = 128 only)."""
         sf = shared_fields
         if any(m == "pa" for m in sf["_sim_info"]["meas_types"]):
             raise NotImplementedError("'pa' toy measurements are not simulations; not on the CUDA path")
@@ -86,6 +87,8 @@ class PathCache:
         if kernel == "seulex":
             _capi.check_extrapolation_problem(sf.get("model", "std"), sf["_sim_info"]["nx"])
             self.flags |= _capi.OPT_EXTRAPOLATION | _capi.OPT_CTA_PER_TRAJ
+        elif kernel == "cta":
+            self.flags |= _capi.OPT_CTA_PER_TRAJ
         elif kernel != "warp":
             raise ValueError(f"unknown kernel {kernel!r}")
 

@@ -66,3 +66,21 @@ def test_pa_measurements_are_refused():
     sf["_sim_info"] = dict(sf["_sim_info"], meas_types=["TRPL", "pa", "TRPL", "TRPL"])
     with pytest.raises(NotImplementedError):
         PathCache(sf, ctx=StubContext())
+
+
+def test_kernel_names_map_to_flags(monkeypatch):
+    """PathCache maps "warp" | "cta" | "seulex" to launch flags; CudaEvaluator reads them back and
+    runs "auto" as "warp"."""
+    from metrotrpl_b200 import metropolis, trial_move_evaluation
+    sf, _ = shared_fields(_T=np.array([1.0, 2.0]))
+    assert PathCache(sf, ctx=StubContext()).flags == 0
+    assert PathCache(sf, ctx=StubContext(), kernel="cta").flags == _capi.OPT_CTA_PER_TRAJ
+    with pytest.raises(ValueError, match="unknown kernel"):
+        PathCache(sf, ctx=StubContext(), kernel="auto")
+    monkeypatch.setattr(trial_move_evaluation, "get_context", lambda device=None: StubContext())
+    for name, kernel, flags, resident in (("auto", "warp", 0, 148 * 8), ("warp", "warp", 0, 148 * 8),
+                                          ("cta", "cta", _capi.OPT_CTA_PER_TRAJ, 148 * 2)):
+        ev = metropolis.CudaEvaluator(sf, kernel=name)
+        assert (ev.kernel, ev.flags, ev._resident) == (kernel, flags | _capi.OPT_LADDER, resident)
+    with pytest.raises(ValueError, match="unknown kernel"):
+        metropolis.CudaEvaluator(sf, kernel="bogus")
