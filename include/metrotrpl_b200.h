@@ -58,11 +58,13 @@ enum trpl_opt_flags { TRPL_OPT_FORCE_MIN_Y = 1, TRPL_OPT_NO_LIKELIHOOD = 2, TRPL
                       TRPL_OPT_CTA_PER_TRAJ = 16, /* one trajectory per CTA of 128 threads instead of one per
                                                     warp: lowest latency per trajectory, for small batches
                                                     (tempering); 'std' model, nx = 128 only */
-                      TRPL_OPT_EXTRAPOLATION = 32 /* integrate with the order-6 extrapolation method
+                      TRPL_OPT_EXTRAPOLATION = 32, /* integrate with the order-6 extrapolation method
                                                     (csrc/extrapolation.h) instead of RODAS4; together with
                                                     TRPL_OPT_CTA_PER_TRAJ its six columns run in parallel on
                                                     the four warps of a CTA: a quarter of the latency per
-                                                    trajectory; 'std' and 'traps' models, nx = 128 only */ };
+                                                    trajectory; 'std' and 'traps' models, nx = 128 only */
+                      TRPL_OPT_FIT = 64 /* also keep the fitted curves: what the likelihood compares, per
+                                          point; see trpl_download_fit */ };
 
 /* one measurement (sim_info["lengths"/"nx"/"meas_types"][i] + its slice of the data arrays) */
 typedef struct trpl_meas_desc {
@@ -144,6 +146,17 @@ int trpl_loglik_batch(trpl_handle* h, int32_t n_sets, const double* params, cons
 /* forward_solver.solve() for a batch: curves only (flags |= TRPL_OPT_NO_LIKELIHOOD). */
 int trpl_solve_batch(trpl_handle* h, int32_t n_sets, const double* params, const double* aux,
                      const trpl_solver_opts* opts, double* curves, int32_t* status, int32_t* nsteps);
+
+/* Fitted curves of the last run, which must have had TRPL_OPT_FIT (with the likelihood and uploaded
+ * vals): fit [n_sets][n_times_total], laid out like curves.  For the trajectory (set s, measurement m),
+ * point k < n_c holds log10(|y_k|) + scale_shift, the left operand of the likelihood's residual
+ * r_k = fit_k - vals_k: y is the simulated signal after the min_y floor (and the TRPL_OPT_FORCE_MIN_Y
+ * floor) or, for a measurement with an IRF, the convolved, max-shifted signal interpolated back onto
+ * the measurement times.  n_c = n_t without IRF; with IRF it is the prefix of times inside the
+ * convolved span.  Points k >= n_c are NaN, and so is the whole slice when the convolution failed
+ * (TRPL_ST_CONV_FAIL).  The fit does not depend on the temperatures or model uncertainties in aux, and
+ * asking for it changes no other output. */
+int trpl_download_fit(trpl_handle* h, double* fit);
 
 /* Split form used for device-resident timing: inputs stay in HBM between runs. */
 int trpl_upload_batch(trpl_handle* h, int32_t n_sets, const double* params, const double* aux);

@@ -30,6 +30,7 @@ INI_IDS = {"density": 0, "fluence": 1}
 ST_MAX_STEPS, ST_H_UNDERFLOW, ST_NONFINITE, ST_FLOORED, ST_NEG_FRAC, ST_NAN_LL, ST_CONV_FAIL = 1, 2, 4, 8, 16, 32, 64
 ST_EXPLICIT = 128
 OPT_FORCE_MIN_Y, OPT_NO_LIKELIHOOD, OPT_LADDER, OPT_NO_EXPLICIT, OPT_CTA_PER_TRAJ, OPT_EXTRAPOLATION = 1, 2, 4, 8, 16, 32
+OPT_FIT = 64      # also keep the fitted curves (Context.download_fit)
 
 # Defaults of the integrator.  RTOL keeps the reference's default value and meaning
 # (forward_solver.py:18).  The reference's default ATOL (1e-10 nm^-3, forward_solver.py:19) is larger
@@ -249,6 +250,7 @@ def load_library() -> C.CDLL:
     lib.trpl_upload_batch.argtypes = [H, C.c_int32, dp, dp]
     lib.trpl_run_resident.argtypes = [H, C.POINTER(SolverOpts), C.c_int32]
     lib.trpl_download_results.argtypes = [H, dp, ip, ip, dp]
+    lib.trpl_download_fit.argtypes = [H, dp]
     lib.trpl_last_kernel_ms.argtypes = [H, C.POINTER(C.c_float)]
     lib.trpl_launch_count.argtypes = [H]
     lib.trpl_launch_count.restype = C.c_int64
@@ -369,6 +371,7 @@ class Context:
         status = np.empty((n_sets, prob.n_meas), dtype=np.int32)
         nsteps = np.empty((n_sets, prob.n_meas, 2), dtype=np.int32)
         curves = np.empty((n_sets, prob.n_times_total)) if want_curves else None
+        self._n_sets = n_sets
         self._check(self.lib.trpl_loglik_batch(
             self.h, n_sets, _ptr(params, C.c_double), _ptr(aux, C.c_double), C.byref(opts),
             _ptr(logll, C.c_double), _ptr(status, C.c_int32), _ptr(nsteps, C.c_int32),
@@ -410,6 +413,15 @@ class Context:
             self.h, _ptr(logll, C.c_double), _ptr(status, C.c_int32), _ptr(nsteps, C.c_int32),
             _ptr(curves, C.c_double)))
         return logll, status, nsteps, curves
+
+    def download_fit(self):
+        """[n_sets, n_times_total] fitted curves of the last run, which had OPT_FIT: per point what the
+        likelihood compared with vals, log10(|signal|) + log10(_s#) after the min_y floor and, with an
+        IRF, after convolution and trim; NaN past the compared points (include/metrotrpl_b200.h,
+        trpl_download_fit)."""
+        fit = np.empty((self._n_sets, self.problem.n_times_total))
+        self._check(self.lib.trpl_download_fit(self.h, _ptr(fit, C.c_double)))
+        return fit
 
     def last_kernel_ms(self) -> float:
         ms = C.c_float()

@@ -209,9 +209,10 @@ TRPL_FN bool irf_convolve_trim(const double* times, const double* curve, int n_t
 
 // Likelihood of a stored signal sol[0..n_c) against vals/uncs[0..n_c): abs/negative count,
 // optional set_min_y floor, log10 residuals, three temperatures (trial_move_evaluation.py:117-166).
+// fit_out (optional): the compared values log10(|sol|, floored) + shift, [n_c].
 TRPL_FN void array_loglik(const double* sol, int n_c, const double* vals, const double* uncs,
                           double shift, const double* s2T, bool force_min_y, double* ll, double& n_neg,
-                          double* r2_out, double* u2_out) {
+                          double* r2_out, double* u2_out, double* fit_out) {
   const ivec lane = lane_id();
   int first_floor = n_c;
   double floor_y = 0.0;
@@ -241,7 +242,9 @@ TRPL_FN void array_loglik(const double* sol, int n_c, const double* vals, const 
     ya = sel(k >= first_floor, floor_y, ya);
     const real vk = gather(vals, k, take, 0.0);
     const real uk = gather(uncs, k, take, 1.0);
-    const real r = (vlog10(ya) + shift) - vk;
+    const real f = vlog10(ya) + shift;
+    if (fit_out) scatter(fit_out, k, take, f);
+    const real r = f - vk;
     const real r2 = r * r;
     const real u2 = 2.0 * (uk * uk);
     l0 = l0 + sel(take, r2 * rcp(s2T[0] + u2), 0.0);

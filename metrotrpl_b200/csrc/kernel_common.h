@@ -58,6 +58,7 @@ struct KernelArgs {
   int n_traj, n_meas, n_times_total;
   int slots_per_cta;         // trajectories a CTA runs at once (warps, teams or 1): step-log / scratch slices
   SolverOpts opt;
+  double* fit;               // [n_sets][n_times_total] fitted curves (TRPL_OPT_FIT, trpl_fit_kernel) or null
 };
 
 // Queue position -> trajectory index (results are indexed [set][meas]).  Without an explicit order

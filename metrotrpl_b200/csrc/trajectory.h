@@ -86,7 +86,7 @@ enum StatusBits {
 };
 
 enum OptFlags { OPT_FORCE_MIN_Y = 1, OPT_NO_LIKELIHOOD = 2, OPT_LADDER = 4, OPT_NO_EXPLICIT = 8, OPT_CTA_PER_TRAJ = 16,
-                OPT_EXTRAPOLATION = 32 };
+                OPT_EXTRAPOLATION = 32, OPT_FIT = 64 };
 
 struct SolverOpts {
   double rtol, atol;
@@ -944,7 +944,7 @@ TRPL_FN void finalize_trajectory(const TrajIn& in, const TailIn& tl, const Solve
       }
       if (ok) array_loglik(sol, n_c, in.vals, in.uncs, in.scale_shift, in.s2T,
                            (opt.flags & OPT_FORCE_MIN_Y) != 0, l, n_neg,
-                           ladder ? tl.r2_scratch : nullptr, ladder ? tl.u2_scratch : nullptr);
+                           ladder ? tl.r2_scratch : nullptr, ladder ? tl.u2_scratch : nullptr, nullptr);
     } else {
       l[0] = mid.l[0]; l[1] = mid.l[1]; l[2] = mid.l[2];
       n_neg = mid.n_neg;
@@ -967,6 +967,37 @@ TRPL_FN void finalize_trajectory(const TrajIn& in, const TailIn& tl, const Solve
   } else {
     out.logll[0] = out.logll[1] = out.logll[2] = 0.0;
   }
+}
+
+// ---- fitted curve (OPT_FIT): what the likelihood compared, point by point ----------------------
+// From the trajectory's stored signal (in.curve, complete once its trajectory kernel is done), by
+// the routines finalize_trajectory uses: the IRF convolution and trim, then array_loglik, which
+// writes log10(|y|, floored) + scale_shift for the n_c compared points.  The streaming sums of
+// emitter_accumulate form the same value from the same y (the curve holds it bit for bit, with the
+// min_y floor applied), so fit[k] - vals[k] is the residual of every path.  Points past n_c are
+// NaN; all of them when the convolution failed.  Run as its own pass so that nothing of it is
+// compiled into the trajectory kernels.
+TRPL_FN void fit_trajectory(const TrajIn& in, const TailIn& tl, const SolverOpts& opt, double* fit) {
+  const int n_t = in.md->n_t;
+  int n_c = n_t;
+  bool ok = true;
+  const double* sol = in.curve;
+  if (tl.irf.nk > 0) {
+    ok = irf_convolve_trim(in.times, in.curve, n_t, tl.irf, n_c);
+    sol = tl.irf.trim;
+  }
+  if (!ok) n_c = 0;
+  if (n_c > 0) {
+    double l[3], n_neg;
+    array_loglik(sol, n_c, in.vals, in.uncs, in.scale_shift, in.s2T, (opt.flags & OPT_FORCE_MIN_Y) != 0, l, n_neg,
+                 nullptr, nullptr, fit);
+  }
+  const ivec lane = lane_id();
+  for (int k0 = n_c; k0 < n_t; k0 += LANES) {
+    const ivec k = iadd(lane, k0);
+    scatter(fit, k, k < n_t, splat(NAN));
+  }
+  warp_sync();
 }
 
 }  // namespace trpl

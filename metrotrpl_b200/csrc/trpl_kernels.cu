@@ -149,6 +149,26 @@ __global__ void __launch_bounds__(cta::NX, 2) trpl_cta_kernel(const KernelArgs a
   }
 }
 
+// TRPL_OPT_FIT: the fitted curve of every trajectory (trajectory.h fit_trajectory), from the curves
+// the trajectory kernel stored.  Runs after it on the same stream, one warp per CTA, each CTA in its
+// own scratch slice (launched with at most as many CTAs as the trajectory kernel had slices).  The
+// convolution is set up as in finish_traj.
+__global__ void __launch_bounds__(32) trpl_fit_kernel(const KernelArgs a) {
+  double* ws = a.scratch ? a.scratch + (size_t)blockIdx.x * a.scratch_stride : nullptr;
+  for (int traj = blockIdx.x; traj < a.n_traj; traj += gridDim.x) {
+    TrajIn in;
+    setup_traj(a, traj, 0, in);
+    const MeasDesc* md = in.md;
+    TailIn tl;
+    tl.irf.nk = (a.irf_mom && ws && md->irf_nk > 0) ? md->irf_nk : 0;
+    tl.irf.dt = md->irf_dt;
+    tl.irf.mom = a.irf_mom ? a.irf_mom + 3 * (size_t)md->irf_off : nullptr;
+    tl.irf.ry = ws; tl.irf.hk = ws ? ws + a.off_hk : nullptr; tl.irf.trim = ws ? ws + a.off_trim : nullptr;
+    const int set = traj / a.n_meas;
+    fit_trajectory(in, tl, a.opt, a.fit + (size_t)set * a.n_times_total + in.md->t_off);
+  }
+}
+
 // Replica exchange needs each chain's likelihood at every ladder temperature summed over its
 // measurements (the reference sums ll_func[ss](T) over ss, metropolis.py:73-76): [n_sets][n_temps].
 // NaN (a failed curve) becomes -inf, as eval_trial_move's callers treat it.
@@ -222,6 +242,8 @@ struct trpl_handle {
   int queue_n = 0;           // trajectories the explicit queue order is for (0: none)
   int n_sets = 0;
   bool curves_valid = false;
+  DevBuf<double> d_fit;
+  bool fit_valid = false;
   float last_ms = 0.f;
   int64_t launches = 0;
 };
@@ -280,6 +302,13 @@ int run_plan(trpl_handle* h, KernelArgs a, const LaunchPlan& p, const char* what
   for (const void* k : {p.kernel, two_pass ? p.explicit_kernel : nullptr}) {
     if (!k) continue;
     CU(cudaLaunchKernel(k, grid, p.block, args, p.smem, h->stream));
+    h->launches += 1;
+  }
+  if (a.fit) {
+    KernelArgs f = a;
+    f.slots_per_cta = 1;
+    void* fargs[] = {&f};
+    CU(cudaLaunchKernel((const void*)trpl_fit_kernel, grid * p.traj_per_cta, 32, fargs, 0, h->stream));
     h->launches += 1;
   }
   CU(cudaEventRecord(h->ev1, h->stream));
@@ -632,6 +661,11 @@ int trpl_run_resident(trpl_handle* h, const trpl_solver_opts* opts, int32_t want
   if (h->n_sets < 1) return fail("no batch uploaded");
   if (!(opts->rtol > 0) || !(opts->atol >= 0) || opts->max_steps < 1) return fail("bad solver options");
   const bool want_ll = !(opts->flags & TRPL_OPT_NO_LIKELIHOOD);
+  const bool want_fit = (opts->flags & TRPL_OPT_FIT) != 0;
+  h->fit_valid = false;
+  if (want_fit && !want_ll)
+    return fail("TRPL_OPT_FIT returns what the likelihood compares: it cannot be combined with TRPL_OPT_NO_LIKELIHOOD");
+  if (want_fit && !h->have_vals) return fail("TRPL_OPT_FIT needs measurement values (vals, uncs in trpl_set_problem)");
   if (want_ll && !h->have_vals) return fail("likelihood requested but no measurement values uploaded");
   if (opts->flags & TRPL_OPT_FORCE_MIN_Y) want_curves = 1;   // the min_y pass re-reads the curve
   const bool conv = want_ll && h->any_irf;
@@ -640,6 +674,7 @@ int trpl_run_resident(trpl_handle* h, const trpl_solver_opts* opts, int32_t want
   const bool ladder = want_ll && (opts->flags & TRPL_OPT_LADDER);
   if (ladder && h->n_ladder < 1) return fail("TRPL_OPT_LADDER without trpl_set_ladder");
   if (ladder) want_curves = 1;
+  if (want_fit) want_curves = 1;           // the fit pass reads the stored curves
   CU(cudaSetDevice(h->device));
   KernelArgs a;
   a.params = h->d_params.p; a.aux = h->d_aux.p; a.meas = h->d_meas.p; a.times = h->d_times.p;
@@ -672,6 +707,12 @@ int trpl_run_resident(trpl_handle* h, const trpl_solver_opts* opts, int32_t want
     a.ladder_T = h->d_ladder_T.p; a.ladder_out = h->d_ladder_out.p; a.n_ladder = h->n_ladder;
     h->ladder_valid = true;
   }
+  a.fit = nullptr;
+  if (want_fit) {
+    CU(h->d_fit.reserve((size_t)h->n_sets * h->n_times_total));
+    a.fit = h->d_fit.p;
+    h->fit_valid = true;
+  }
   a.counter = h->d_counter.p;
   a.meas_order = h->d_order.p;
   a.queue = (h->queue_n > 0 && h->queue_n == h->n_sets * h->n_meas) ? h->d_queue.p : nullptr;
@@ -685,6 +726,16 @@ int trpl_run_resident(trpl_handle* h, const trpl_solver_opts* opts, int32_t want
 #else
   return launch_npl<MODEL_TRAPS>(h, a);
 #endif
+}
+
+int trpl_download_fit(trpl_handle* h, double* fit) {
+  if (!h || !fit) return fail("null argument");
+  if (!h->fit_valid) return fail("the last run did not produce fitted curves (run with TRPL_OPT_FIT)");
+  CU(cudaSetDevice(h->device));
+  CU(cudaMemcpyAsync(fit, h->d_fit.p, sizeof(double) * (size_t)h->n_sets * h->n_times_total, cudaMemcpyDeviceToHost,
+                     h->stream));
+  CU(cudaStreamSynchronize(h->stream));
+  return 0;
 }
 
 int trpl_download_results(trpl_handle* h, double* logll, int32_t* status, int32_t* nsteps, double* curves) {

@@ -10,7 +10,7 @@ host only packs parameters and reads back one scalar per (state, measurement, te
 """
 from __future__ import annotations
 
-from dataclasses import dataclass
+from dataclasses import dataclass, field
 from typing import Optional, Sequence
 
 import numpy as np
@@ -28,10 +28,26 @@ class BatchLikelihood:
     status: np.ndarray       # [n_sets, n_meas]
     nsteps: np.ndarray       # [n_sets, n_meas, 2]
     curves: Optional[np.ndarray] = None
+    fit: Optional[np.ndarray] = None        # [n_sets, n_times_total] fitted curves (want_fit=True)
+    problem: Optional[_capi.PackedProblem] = field(default=None, repr=False)   # for fitted()
 
     def at_temperature(self, slot: int) -> np.ndarray:
         """Sum over measurements at temperature slot 0..2 (the ll_funcs of the reference)."""
         return self.per_meas[:, :, slot].sum(axis=1)
+
+    def fitted(self, m: int, s: int = 0):
+        """(times, fit, vals, uncs) of measurement m for parameter set s, cut to the points the
+        likelihood compared: fit - vals are its residuals, log10(model) - log10(data).  Without an IRF
+        that is every point; with one, the times inside the convolved span.  Empty when the
+        convolution failed.  Needs eval_trial_moves(..., want_fit=True)."""
+        if self.fit is None:
+            raise ValueError("no fitted curves: evaluate with want_fit=True")
+        prob = self.problem
+        sl = slice(int(prob.t_off[m]), int(prob.t_off[m] + prob.n_t[m]))
+        f = self.fit[s, sl]
+        done = np.flatnonzero(~np.isnan(f))
+        n_c = int(done[-1]) + 1 if done.size else 0        # compared points are a prefix; NaN after it
+        return prob.times[sl][:n_c], f[:n_c], prob.vals[sl][:n_c], prob.uncs[sl][:n_c]
 
 
 class PathCache:
@@ -128,10 +144,12 @@ class PathCache:
 
 
 def eval_trial_moves(states, temps, sigmas, shared_fields, cache: Optional[PathCache] = None,
-                     want_curves=False, honor_hmax=False) -> BatchLikelihood:
+                     want_curves=False, honor_hmax=False, want_fit=False) -> BatchLikelihood:
     """Log-likelihood of many proposed states in one launch.
 
     temps : [n_sets] (own temperature) or [n_sets, 3] (own + two others, e.g. the swap partners').
+    want_fit : also return the fitted curves, what the likelihood compared with the data point by
+        point (BatchLikelihood.fit, BatchLikelihood.fitted); no other result changes.
     """
     if cache is None:
         cache = PathCache(shared_fields)
@@ -142,11 +160,14 @@ def eval_trial_moves(states, temps, sigmas, shared_fields, cache: Optional[PathC
         temps = np.repeat(temps[:, None], 3, axis=1)
     params, aux = cache.pack(states, sigmas, temps)
     cache.ctx.set_problem_if_needed(cache.prob)
-    per, status, nsteps, curves = cache.ctx.loglik_batch(params, aux, cache.opts(honor_hmax),
-                                                         want_curves=want_curves)
+    opts = cache.opts(honor_hmax)
+    if want_fit:
+        opts.flags |= _capi.OPT_FIT
+    per, status, nsteps, curves = cache.ctx.loglik_batch(params, aux, opts, want_curves=want_curves)
+    fit = cache.ctx.download_fit() if want_fit else None
     logll = per[:, :, 0].sum(axis=1)
     logll = np.where(np.isnan(logll), -np.inf, logll)
-    return BatchLikelihood(logll, per, status, nsteps, curves)
+    return BatchLikelihood(logll, per, status, nsteps, curves, fit, cache.prob if want_fit else None)
 
 
 def eval_trial_move(state, unique_fields, shared_fields, logger=None, cache=None):
