@@ -27,6 +27,9 @@ struct IrfDesc {
   double* trim;        // scratch: convolved curve on the measurement times [n_t]
 };
 
+// points of a curve ending at tend resampled to dt/2: len(np.arange(0, tend + dt/4, dt/2))
+TRPL_HD int irf_resample_count(double tend, double dt) { return (int)ceil((tend + dt / 4) / (dt / 2)); }
+
 // np.interp(x, xp, fp) for one x per lane, xp ascending, xp[0] <= x <= xp[n-1]
 TRPL_FN real interp_lanes(const double* xp, const double* fp, int n, const real& x, const mask& take) {
   ivec lo = isplat(0);
@@ -70,7 +73,7 @@ TRPL_FN bool irf_convolve_trim(const double* times, const double* curve, int n_t
   const ivec lane = lane_id();
   const double tend = times[n_t - 1];
   const double half = f.dt / 2;
-  const int n_rs = (int)ceil((tend + f.dt / 4) / half);      // len(np.arange(0, tend + dt/4, dt/2))
+  const int n_rs = irf_resample_count(tend, f.dt);
   if (n_rs < 3) return false;
   const int nk = (n_rs - 1) / 2;
   const int last_rs = n_rs - 1;

@@ -34,6 +34,7 @@
 // device
 // ------------------------------------------------------------------------------------------
 #define TRPL_FN __device__ __forceinline__
+#define TRPL_HD __host__ __device__ __forceinline__     // also called by the library's host code
 #define TRPL_UNROLL _Pragma("unroll")
 #define TRPL_UNROLL4 _Pragma("unroll 4")
 
@@ -402,6 +403,7 @@ template <int N> TRPL_FN void mem_st_pairs(const LaneTm& m, int p, const real* v
 #include <stdio.h>
 #include <stdlib.h>
 #define TRPL_FN inline
+#define TRPL_HD inline
 #define TRPL_UNROLL
 #define TRPL_UNROLL4
 

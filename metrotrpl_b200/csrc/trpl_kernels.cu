@@ -45,14 +45,14 @@ __global__ void __launch_bounds__(32 * WARPS_PER_CTA, CTAS_PER_SM) trpl_forward_
     if (q >= a.n_traj) break;
     const int traj = queue_traj(a, q);
     TrajIn in;
-    setup_traj(a, traj, warp, in);
+    setup_traj(a, traj, cta_slot(a, warp), in);
     TrajOut out;
     TrajMid mid;
     if (run_trajectory<NPL, MODEL, FULL>(in, a.opt, mem, out, mid, allow_defer)) {
       if (lane == 0) a.defer_list[atomicAdd(a.defer_count, 1)] = traj;     // non-stiff: explicit path
       continue;
     }
-    finish_traj(a, traj, warp, in, mid, out);
+    finish_traj(a, traj, cta_slot(a, warp), in, mid, out);
   }
   tmem_release<SL>(warp, mem.tm);
 }
@@ -71,12 +71,12 @@ __global__ void __launch_bounds__(32 * WARPS_PER_CTA, CTAS_PER_SM) trpl_explicit
     if (q >= n) break;
     const int traj = a.defer_list[q];
     TrajIn in;
-    setup_traj(a, traj, warp, in);
+    setup_traj(a, traj, cta_slot(a, warp), in);
     TrajOut out;
     TrajMid mid;
     run_trajectory_explicit<NPL, MODEL, FULL>(in, a.opt, mem, out, mid);
     out.status |= ST_EXPLICIT;
-    finish_traj(a, traj, warp, in, mid, out);
+    finish_traj(a, traj, cta_slot(a, warp), in, mid, out);
   }
   tmem_release<SL>(warp, mem.tm);
 }
@@ -96,11 +96,11 @@ __global__ void __launch_bounds__(32 * WARPS_PER_CTA, CTAS_PER_SM) trpl_seulex_k
     if (q >= a.n_traj) break;
     const int traj = queue_traj(a, q);
     TrajIn in;
-    setup_traj(a, traj, warp, in);
+    setup_traj(a, traj, cta_slot(a, warp), in);
     TrajOut out;
     TrajMid mid;
     run_trajectory_seulex<NPL, MODEL, FULL>(in, a.opt, mem, out, mid);
-    finish_traj(a, traj, warp, in, mid, out);
+    finish_traj(a, traj, cta_slot(a, warp), in, mid, out);
   }
   tmem_release<SL>(warp, mem.tm);
 }
@@ -123,11 +123,11 @@ __global__ void __launch_bounds__(32 * WARPS_PER_CTA, CTAS_PER_SM) trpl_seulex_c
     if (q >= a.n_traj) break;
     const int traj = queue_traj(a, q);
     TrajIn in;
-    setup_traj(a, traj, 0, in);               // slots_per_cta == 1: one step log / scratch slice per CTA
+    setup_traj(a, traj, cta_slot(a, 0), in);    // slots_per_cta == 1: one step log / scratch slice per CTA
     TrajOut out;
     TrajMid mid;
     run_trajectory_seulex_cta<NPL, MODEL, FULL>(in, a.opt, mem, xch, &s_flag, warp, out, mid);
-    if (warp == 0) finish_traj(a, traj, 0, in, mid, out);
+    if (warp == 0) finish_traj(a, traj, cta_slot(a, 0), in, mid, out);
   }
   tmem_release<SL>(warp, mem.tm);
 }
@@ -141,23 +141,23 @@ __global__ void __launch_bounds__(cta::NX, 2) trpl_cta_kernel(const KernelArgs a
     if (q >= a.n_traj) break;
     const int traj = queue_traj(a, q);
     TrajIn in;
-    setup_traj(a, traj, 0, in);
+    setup_traj(a, traj, cta_slot(a, 0), in);
     TrajOut out;
     TrajMid mid;
     cta::run_trajectory_cta(in, a.opt, s, out, mid);
-    if (threadIdx.x < 32) finish_traj(a, traj, 0, in, mid, out);
+    if (threadIdx.x < 32) finish_traj(a, traj, cta_slot(a, 0), in, mid, out);
   }
 }
 
 // TRPL_OPT_FIT: the fitted curve of every trajectory (trajectory.h fit_trajectory), from the curves
 // the trajectory kernel stored.  Runs after it on the same stream, one warp per CTA, each CTA in its
 // own scratch slice (launched with at most as many CTAs as the trajectory kernel had slices).  The
-// convolution is set up as in finish_traj.
+// convolution is set up as in tail_in, with the CTA's slice formed once, before the loop.
 __global__ void __launch_bounds__(32) trpl_fit_kernel(const KernelArgs a) {
   double* ws = a.scratch ? a.scratch + (size_t)blockIdx.x * a.scratch_stride : nullptr;
   for (int traj = blockIdx.x; traj < a.n_traj; traj += gridDim.x) {
     TrajIn in;
-    setup_traj(a, traj, 0, in);
+    setup_traj(a, traj, blockIdx.x, in);
     const MeasDesc* md = in.md;
     TailIn tl;
     tl.irf.nk = (a.irf_mom && ws && md->irf_nk > 0) ? md->irf_nk : 0;
@@ -524,8 +524,7 @@ int trpl_set_problem(trpl_handle* h, int32_t model, int32_t n_meas, const trpl_m
     if ((size_t)m.n_t > h->max_nt) h->max_nt = m.n_t;
     if (m.irf_nk > 0) {
       h->any_irf = true;
-      const double tend = times[m.t_off + m.n_t - 1];
-      const size_t n_rs = (size_t)ceil((tend + m.irf_dt / 4) / (m.irf_dt / 2));
+      const size_t n_rs = irf_resample_count(times[m.t_off + m.n_t - 1], m.irf_dt);
       if (n_rs > h->max_nrs) h->max_nrs = n_rs;
       if (m.irf_off + m.irf_nk > h->irf_rows_needed) h->irf_rows_needed = m.irf_off + m.irf_nk;
     }
@@ -660,59 +659,24 @@ int trpl_run_resident(trpl_handle* h, const trpl_solver_opts* opts, int32_t want
   if (!h || !opts) return fail("null argument");
   if (h->n_sets < 1) return fail("no batch uploaded");
   if (!(opts->rtol > 0) || !(opts->atol >= 0) || opts->max_steps < 1) return fail("bad solver options");
-  const bool want_ll = !(opts->flags & TRPL_OPT_NO_LIKELIHOOD);
-  const bool want_fit = (opts->flags & TRPL_OPT_FIT) != 0;
   h->fit_valid = false;
-  if (want_fit && !want_ll)
-    return fail("TRPL_OPT_FIT returns what the likelihood compares: it cannot be combined with TRPL_OPT_NO_LIKELIHOOD");
-  if (want_fit && !h->have_vals) return fail("TRPL_OPT_FIT needs measurement values (vals, uncs in trpl_set_problem)");
-  if (want_ll && !h->have_vals) return fail("likelihood requested but no measurement values uploaded");
-  if (opts->flags & TRPL_OPT_FORCE_MIN_Y) want_curves = 1;   // the min_y pass re-reads the curve
-  const bool conv = want_ll && h->any_irf;
-  if (conv && !h->have_irf) return fail("measurements ask for IRF convolution but trpl_set_irf was not called");
-  if (conv) want_curves = 1;
-  const bool ladder = want_ll && (opts->flags & TRPL_OPT_LADDER);
-  if (ladder && h->n_ladder < 1) return fail("TRPL_OPT_LADDER without trpl_set_ladder");
-  if (ladder) want_curves = 1;
-  if (want_fit) want_curves = 1;           // the fit pass reads the stored curves
+  RunPlan p;
+  const ProblemFacts pf{h->have_vals, h->any_irf, h->have_irf, h->n_ladder, h->max_nrs, h->max_nt};
+  if (const char* why = plan_run(pf, opts->flags, want_curves != 0, p)) return fail(why);
   CU(cudaSetDevice(h->device));
+  if (p.curves) CU(h->d_curves.reserve((size_t)h->n_sets * h->n_times_total));
+  h->curves_valid = p.curves;
+  h->ladder_valid = false;
+  if (p.ladder) CU(h->d_ladder_out.reserve((size_t)h->n_sets * h->n_meas * h->n_ladder));
+  h->ladder_valid = p.ladder;
+  if (p.fit) CU(h->d_fit.reserve((size_t)h->n_sets * h->n_times_total));
+  h->fit_valid = p.fit;
   KernelArgs a;
   a.params = h->d_params.p; a.aux = h->d_aux.p; a.meas = h->d_meas.p; a.times = h->d_times.p;
   a.vals = h->have_vals ? h->d_vals.p : nullptr; a.uncs = h->have_vals ? h->d_uncs.p : nullptr;
   a.profiles = h->have_profiles ? h->d_profiles.p : nullptr;
   a.logll = h->d_logll.p; a.status = h->d_status.p; a.nsteps = h->d_nsteps.p;
-  a.curves = nullptr;
-  if (want_curves) {
-    CU(h->d_curves.reserve((size_t)h->n_sets * h->n_times_total));
-    a.curves = h->d_curves.p;
-  }
-  h->curves_valid = want_curves != 0;
-  a.irf_mom = nullptr; a.scratch = nullptr; a.scratch_stride = 0; a.off_hk = 0; a.off_trim = 0;
-  a.off_r2 = 0; a.off_u2 = 0; a.ladder_T = nullptr; a.ladder_out = nullptr; a.n_ladder = 0;
-  h->ladder_valid = false;
-  if (conv || ladder) {
-    // per-warp scratch: resampled | convolved | trimmed curve | residuals^2 | 2 unc^2 (all stay in L2)
-    const size_t nrs = conv ? h->max_nrs : 0;
-    const size_t n_hk = conv ? (h->max_nrs - 1) / 2 + 1 : 0;
-    const size_t nt4 = (h->max_nt + 3) & ~(size_t)3;
-    a.off_hk = (nrs + 3) & ~(size_t)3;
-    a.off_trim = a.off_hk + ((n_hk + 3) & ~(size_t)3);
-    a.off_r2 = a.off_trim + nt4;
-    a.off_u2 = a.off_r2 + nt4;
-    a.scratch_stride = a.off_u2 + nt4;        // run_plan sizes the slices and sets a.scratch
-    if (conv) a.irf_mom = h->d_irf.p;
-  }
-  if (ladder) {
-    CU(h->d_ladder_out.reserve((size_t)h->n_sets * h->n_meas * h->n_ladder));
-    a.ladder_T = h->d_ladder_T.p; a.ladder_out = h->d_ladder_out.p; a.n_ladder = h->n_ladder;
-    h->ladder_valid = true;
-  }
-  a.fit = nullptr;
-  if (want_fit) {
-    CU(h->d_fit.reserve((size_t)h->n_sets * h->n_times_total));
-    a.fit = h->d_fit.p;
-    h->fit_valid = true;
-  }
+  p.set_args(a, h->d_curves.p, h->d_irf.p, h->d_ladder_T.p, h->d_ladder_out.p, h->n_ladder, h->d_fit.p);
   a.counter = h->d_counter.p;
   a.meas_order = h->d_order.p;
   a.queue = (h->queue_n > 0 && h->queue_n == h->n_sets * h->n_meas) ? h->d_queue.p : nullptr;

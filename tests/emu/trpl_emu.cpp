@@ -1,101 +1,72 @@
 // trpl_emu.cpp - host lock-step build of the SAME integrator source the CUDA kernel compiles
 // (metrotrpl_b200/csrc/trajectory.h) with TRPL_HOST_EMU.  Test infrastructure only: it lets the
 // CPU-only test tier exercise the warp algorithm (partition + PCR solve, RODAS4 controller, Hermite
-// readout, likelihood) against the oracle.  It is built and loaded by tests/ only and is never
-// reachable from the metrotrpl_b200 package.
+// readout, likelihood) against the oracle.  A run is planned, set up and written back by the
+// library's own code (traj_io.h): the same stored outputs, the same per-slot scratch layout, one slot
+// per OpenMP thread.  It is built and loaded by tests/ only and is never reachable from the
+// metrotrpl_b200 package.
 #define TRPL_HOST_EMU 1
+#include <omp.h>
 #include <stdint.h>
 #include <string.h>
+#include <algorithm>
 #include <vector>
-#include "../../include/metrotrpl_b200.h"
-#include "../../metrotrpl_b200/csrc/trajectory.h"
+#include "../../metrotrpl_b200/csrc/traj_io.h"
 #include "../../metrotrpl_b200/csrc/explicit.h"
 #if TRPL_TEAM == 1
 #include "../../metrotrpl_b200/csrc/extrapolation.h"
 #endif
 
-using namespace trpl;
-
 template <int NPL, int MODEL, bool FULL>
-static void run_all(int n_meas, const MeasDesc* meas, int n_times_total, const double* times,
-                    const double* vals, const double* uncs, const double* profiles, int n_sets,
-                    const double* params, const double* aux, const SolverOpts& opt, double* logll,
-                    int32_t* status, int32_t* nsteps, double* curves, const double* irf_mom,
-                    const double* ladder_T, int n_ladder, double* ladder_out) {
-  const int n_traj = n_sets * n_meas;
-#pragma omp parallel for schedule(dynamic, 1)
-  for (int traj = 0; traj < n_traj; ++traj) {
-    const int set = traj / n_meas, mi = traj % n_meas;
-    const MeasDesc* md = meas + mi;
-    TrajMem sm{simt::LaneMem(Slots<NPL, MODEL>::COUNT), simt::LaneTm(Slots<NPL, MODEL>::TM_COUNT)};
-    TrajIn in;
-    in.par = params + (size_t)set * TRPL_NPARAM;
-    in.md = md;
-    in.times = times + md->t_off;
-    in.vals = vals ? vals + md->t_off : nullptr;
-    in.uncs = uncs ? uncs + md->t_off : nullptr;
-    in.profile = profiles ? profiles + md->prof_off : nullptr;
-    const double* ax = aux + (size_t)traj * TRPL_NAUX;
-    in.scale_shift = ax[TRPL_A_SCALE_SHIFT];
-    in.s2T[0] = ax[TRPL_A_S2T0]; in.s2T[1] = ax[TRPL_A_S2T1]; in.s2T[2] = ax[TRPL_A_S2T2];
-    in.fl_mult = ax[TRPL_A_FLUENCE_MULT]; in.al_mult = ax[TRPL_A_ABSORB_MULT];
-    in.curve = curves ? curves + (size_t)set * n_times_total + md->t_off : nullptr;
-    std::vector<double> hist(3 * HIST_CAP);
-    in.hist = hist.data();
-    const bool want_ll = !(opt.flags & OPT_NO_LIKELIHOOD);
-    const bool conv = irf_mom && md->irf_nk > 0;
-    const bool ladder = (opt.flags & OPT_LADDER) && n_ladder > 0;
-    in.post_pass = want_ll && in.curve && ((opt.flags & OPT_FORCE_MIN_Y) || conv || ladder);
-    TrajOut out;
-    TrajMid mid;
+static void run_all(const KernelArgs& a) {
+#pragma omp parallel
+  {
+    const unsigned slot = omp_get_thread_num();
+#pragma omp for schedule(dynamic, 1)
+    for (int traj = 0; traj < a.n_traj; ++traj) {
+      TrajMem sm{simt::LaneMem(Slots<NPL, MODEL>::COUNT), simt::LaneTm(Slots<NPL, MODEL>::TM_COUNT)};
+      TrajIn in;
+      setup_traj(a, traj, slot, in);
+      TrajOut out;
+      TrajMid mid;
 #if TRPL_TEAM == 1
-    if (opt.flags & OPT_EXTRAPOLATION) {
-      run_trajectory_seulex<NPL, MODEL, FULL>(in, opt, sm, out, mid);      // the one-warp driver
-    } else
+      if (a.opt.flags & OPT_EXTRAPOLATION) {
+        run_trajectory_seulex<NPL, MODEL, FULL>(in, a.opt, sm, out, mid);      // the one-warp driver
+      } else
 #endif
-    if (run_trajectory<NPL, MODEL, FULL>(in, opt, sm, out, mid, !(opt.flags & OPT_NO_EXPLICIT))) {
-      run_trajectory_explicit<NPL, MODEL, FULL>(in, opt, sm, out, mid);
-      out.status |= ST_EXPLICIT;
+      if (run_trajectory<NPL, MODEL, FULL>(in, a.opt, sm, out, mid, !(a.opt.flags & OPT_NO_EXPLICIT))) {
+        run_trajectory_explicit<NPL, MODEL, FULL>(in, a.opt, sm, out, mid);
+        out.status |= ST_EXPLICIT;
+      }
+      TailIn tl;
+      tail_in(a, in, traj, slot, tl);
+      finalize_trajectory(in, tl, a.opt, mid, out);
+      store_result(a, traj, out);
     }
-    std::vector<double> ry, hk, trim;
-    TailIn tl;
-    tl.irf.nk = conv ? md->irf_nk : 0;
-    tl.irf.dt = md->irf_dt;
-    tl.irf.mom = irf_mom ? irf_mom + 3 * (size_t)md->irf_off : nullptr;
-    if (tl.irf.nk > 0) {
-      const double tend = in.times[md->n_t - 1];
-      const size_t n_rs = (size_t)ceil((tend + md->irf_dt / 4) / (md->irf_dt / 2));
-      ry.resize(n_rs + 4); hk.resize(n_rs / 2 + 4); trim.resize(md->n_t + 4);
+    // the fit pass reads the curves of every trajectory: after the loop's closing barrier
+    if (a.fit) {
+#pragma omp for schedule(dynamic, 1)
+      for (int traj = 0; traj < a.n_traj; ++traj) {
+        TrajIn in;
+        setup_traj(a, traj, slot, in);
+        TailIn tl;
+        tail_in(a, in, traj, slot, tl);
+        fit_trajectory(in, tl, a.opt, a.fit + (size_t)(traj / a.n_meas) * a.n_times_total + in.md->t_off);
+      }
     }
-    tl.irf.ry = ry.data(); tl.irf.hk = hk.data(); tl.irf.trim = trim.data();
-    std::vector<double> r2(md->n_t + 4), u2(md->n_t + 4);
-    tl.r2_scratch = ladder ? r2.data() : nullptr; tl.u2_scratch = ladder ? u2.data() : nullptr;
-    tl.ladder_T = ladder_T; tl.ladder_n = n_ladder;
-    tl.ladder_out = ladder_out ? ladder_out + (size_t)traj * n_ladder : nullptr;
-    finalize_trajectory(in, tl, opt, mid, out);
-    for (int k = 0; k < 3; ++k) logll[3 * (size_t)traj + k] = out.logll[k];
-    status[traj] = out.status;
-    if (nsteps) { nsteps[2 * traj] = out.n_acc; nsteps[2 * traj + 1] = out.n_rej; }
   }
 }
 
 template <int MODEL>
-static int dispatch(int max_nx, int n_meas, const MeasDesc* meas, int n_times_total,
-                    const double* times, const double* vals, const double* uncs,
-                    const double* profiles, int n_sets, const double* params, const double* aux,
-                    const SolverOpts& opt, double* logll, int32_t* status, int32_t* nsteps,
-                    double* curves, const double* irf_mom,
-                    const double* ladder_T, int n_ladder, double* ladder_out) {
-#define GO(N, F) run_all<N, MODEL, F>(n_meas, meas, n_times_total, times, vals, uncs, profiles, n_sets, params, aux, opt, logll, status, nsteps, curves, irf_mom, ladder_T, n_ladder, ladder_out)
-  bool all_full = true;
-  for (int i = 0; i < n_meas; ++i) if (meas[i].nx != max_nx) all_full = false;
+static const char* dispatch(int max_nx, bool all_full, const KernelArgs& a) {
+#define GO(N, F) run_all<N, MODEL, F>(a)
 #if TRPL_TEAM >= 2
   // the team vocabularies (team_kernels.cu / team4_kernels.cu): 64 or 128 lanes x 4 nodes, the grids
   // of 129..256 / 257..512 nodes
   constexpr int TOP = 128 * TRPL_TEAM;
   if (all_full && max_nx == TOP) GO(4, true);
   else if (max_nx > TOP / 2 && max_nx <= TOP) GO(4, false);
-  else return 1;
+  else return "nx outside the grids of this team build";
 #else
   // (8 nodes per lane: no product kernel any more, kept for the generic one-warp extrapolation driver)
   if (all_full && max_nx == 128) GO(4, true);
@@ -104,26 +75,53 @@ static int dispatch(int max_nx, int n_meas, const MeasDesc* meas, int n_times_to
   else if (max_nx <= 64) GO(2, false);
   else if (max_nx <= 128) GO(4, false);
   else if (max_nx <= 256) GO(8, false);
-  else return 1;
+  else return "nx > 256 needs a team build";
 #endif
 #undef GO
-  return 0;
+  return nullptr;
 }
 
-extern "C" int trpl_emu_loglik_batch(int32_t model, int32_t n_meas, const trpl_meas_desc* meas,
-                                     int32_t n_times_total, const double* times, const double* vals,
-                                     const double* uncs, const double* profiles, int32_t n_sets,
-                                     const double* params, const double* aux,
-                                     const trpl_solver_opts* opts, double* logll, int32_t* status,
-                                     int32_t* nsteps, double* curves, const double* irf_mom,
-                                     const double* ladder_T, int32_t n_ladder, double* ladder_out) {
+// The library's trpl_set_problem + trpl_set_irf + trpl_set_ladder + trpl_loglik_batch on host arrays:
+// curves, ladder_out and fit are the outputs of the run (null: not wanted).  Returns null, or the
+// message the run is refused with.
+extern "C" const char* trpl_emu_loglik_batch(int32_t model, int32_t n_meas, const trpl_meas_desc* meas,
+                                             int32_t n_times_total, const double* times, const double* vals,
+                                             const double* uncs, const double* profiles, int32_t n_sets,
+                                             const double* params, const double* aux,
+                                             const trpl_solver_opts* opts, double* logll, int32_t* status,
+                                             int32_t* nsteps, double* curves, const double* irf_mom,
+                                             const double* ladder_T, int32_t n_ladder, double* ladder_out,
+                                             double* fit) {
   static_assert(sizeof(trpl_meas_desc) == sizeof(MeasDesc), "ABI struct mismatch");
-  SolverOpts opt;
-  memcpy(&opt, opts, sizeof(opt));
-  int max_nx = 0;
-  for (int i = 0; i < n_meas; ++i) if (meas[i].nx > max_nx) max_nx = meas[i].nx;
   const MeasDesc* md = reinterpret_cast<const MeasDesc*>(meas);
-  if (model == TRPL_MODEL_STD)
-    return dispatch<MODEL_STD>(max_nx, n_meas, md, n_times_total, times, vals, uncs, profiles, n_sets, params, aux, opt, logll, status, nsteps, curves, irf_mom, ladder_T, n_ladder, ladder_out);
-  return dispatch<MODEL_TRAPS>(max_nx, n_meas, md, n_times_total, times, vals, uncs, profiles, n_sets, params, aux, opt, logll, status, nsteps, curves, irf_mom, ladder_T, n_ladder, ladder_out);
+  ProblemFacts pf{vals && uncs, false, irf_mom != nullptr, ladder_T ? n_ladder : 0, 0, 0};
+  int max_nx = 0;
+  for (int i = 0; i < n_meas; ++i) {
+    max_nx = std::max(max_nx, md[i].nx);
+    pf.max_nt = std::max(pf.max_nt, (size_t)md[i].n_t);
+    if (md[i].irf_nk > 0) {
+      pf.any_irf = true;
+      pf.max_nrs = std::max(pf.max_nrs, (size_t)irf_resample_count(times[md[i].t_off + md[i].n_t - 1], md[i].irf_dt));
+    }
+  }
+  bool all_full = true;
+  for (int i = 0; i < n_meas; ++i) if (md[i].nx != max_nx) all_full = false;
+  RunPlan p;
+  if (const char* why = plan_run(pf, opts->flags, curves != nullptr, p)) return why;
+  if ((p.ladder && !ladder_out) || (p.fit && !fit)) return "no output array for the ladder rows or the fit";
+  std::vector<double> own_curves(p.curves && !curves ? (size_t)n_sets * n_times_total : 0);
+  const int n_slots = omp_get_max_threads();
+  std::vector<double> scratch(n_slots * p.scratch_stride), hist((size_t)n_slots * 3 * HIST_CAP);
+  KernelArgs a{};
+  a.params = params; a.aux = aux; a.meas = md; a.times = times;
+  a.vals = pf.have_vals ? vals : nullptr; a.uncs = pf.have_vals ? uncs : nullptr;
+  a.profiles = profiles;
+  a.logll = logll; a.status = status; a.nsteps = nsteps;
+  p.set_args(a, curves ? curves : own_curves.data(), irf_mom, ladder_T, ladder_out, n_ladder, fit);
+  if (p.scratch_stride > 0) a.scratch = scratch.data();
+  a.hist = hist.data();
+  a.n_traj = n_sets * n_meas; a.n_meas = n_meas; a.n_times_total = n_times_total;
+  memcpy(&a.opt, opts, sizeof(SolverOpts));
+  if (model == TRPL_MODEL_STD) return dispatch<MODEL_STD>(max_nx, all_full, a);
+  return dispatch<MODEL_TRAPS>(max_nx, all_full, a);
 }

@@ -217,7 +217,7 @@ def _run_known(backend, guess, lengths, nxs, mtypes, ini, times, vals, uncs, sig
     params = _capi.pack_params(state, idx, units)
     aux = _capi.default_aux(1, len(lengths), [sigma[m] for m in mtypes])
     opts = _capi.make_opts(RTOL=rtol, ATOL=atol, flags=flags)
-    ll, st, ns, cur = backend(prob, params, aux, opts, want_curves or bool(flags & _capi.OPT_FORCE_MIN_Y))
+    ll, st, ns, cur = backend(prob, params, aux, opts, want_curves)
     return ll[0, :, 0], st[0], cur
 
 

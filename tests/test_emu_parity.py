@@ -91,3 +91,28 @@ def test_extrapolation_integrator_closed_forms_and_ragged_inputs():
 
 def test_extrapolation_integrator_traps_model_with_irf_convolution_nx256():
     print(pc.check_traps_irf(_seulex_backend, curve_tol=5e-6))     # measured 1.1e-6 (RODAS4: 3e-7)
+
+
+def test_outputs_without_curves_equal_those_with_curves():
+    """The IRF convolution, the min_y floor and the tempering ladder take the likelihood from the
+    stored curve, so the run stores it whether or not the caller asked for it, as the library's runs
+    do: logll, status, nsteps and ladder rows are bit-identical with and without curves.  traps_irf
+    fixture, first two states."""
+    from metrotrpl_b200 import _capi
+    g = np.load(pc.os.path.join(pc.GOLDEN, "traps_irf.npz"))
+    idx = {str(x): i for i, x in enumerate(g["names"])}
+    sim = {"lengths": list(g["lengths"]), "nx": [int(g["nx"])] * 2, "meas_types": ["TRPL"] * 2, "num_meas": 2}
+    params = _capi.pack_params(g["states"][:2], idx, g["units"], model="traps")
+    aux = _capi.default_aux(2, 2, [1.0] * 2, temps=(1.0, 2.0, 4.0))
+    ladder = np.array([1.0, 3.0, 9.0])
+    for irf, flags in ((True, 0), (False, _capi.OPT_FORCE_MIN_Y), (False, _capi.OPT_LADDER)):
+        prob = _capi.pack_problem(sim, g["inis"], [g["t"]] * 2, list(g["vals"]), list(g["uncs"]), model="traps",
+                                  ini_mode="fluence", irf_convolution=[520, 520] if irf else None,
+                                  irf_tables={520: (g["moments"], g["t_irf"])})
+        lad = ladder if flags & _capi.OPT_LADDER else None
+        opts = _capi.make_opts(RTOL=1e-7, flags=flags)
+        with_curves = emu.loglik_batch(prob, params, aux, opts, True, ladder=lad)
+        without = emu.loglik_batch(prob, params, aux, opts, False, ladder=lad)
+        assert without[3] is None
+        for k in (0, 1, 2) + ((4,) if lad is not None else ()):
+            np.testing.assert_array_equal(without[k], with_curves[k], err_msg=f"irf={irf} flags={flags} output {k}")

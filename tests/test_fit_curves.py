@@ -4,15 +4,16 @@ The fitted curve of a trajectory is, point by point, what the likelihood compare
 log10(|y|) + scale_shift after the min_y floor and, with an IRF, after convolution, max-shift and
 trim; NaN past the compared points.  Checked here against the oracle's restatement of the
 reference's steps applied to the build's own raw curves (exact to rounding) and against the
-log-likelihoods the same run returned.  The host build runs the fit pass on the curves after the run
-(tests/emu/fit_emu.py), as the library does, so it cannot change the run; the GPU tier
-(test_gpu_fit_curves.py, which shares these helpers) checks that no output of the library changes."""
+log-likelihoods the same run returned.  The host build runs the fit pass on the stored curves after
+the run (emu.loglik_batch(..., fit=True)), as the library does, so it cannot change the run; the GPU
+tier (test_gpu_fit_curves.py, which shares these helpers) checks that no output of the library
+changes."""
 import numpy as np
 
 from metrotrpl_b200 import _capi
 from oracle import trpl_oracle as orc
 from tests import parity_cases as pc
-from tests.emu import fit_emu
+from tests.emu import emu
 from tests.test_extrapolation_traps import traps128_problem
 
 # fitted values vs the oracle's steps on the same raw curve: 1e-14 absolute, or two units in the last
@@ -85,7 +86,7 @@ def assert_no_side_effects(with_fit, without_fit):
 
 def emu_run(prob, params, aux, flags, rtol=1e-7):
     """(logll, status, nsteps, curves, fit) of the host build."""
-    return fit_emu.loglik_batch(prob, params, aux, _capi.make_opts(RTOL=rtol, flags=flags))
+    return emu.loglik_batch(prob, params, aux, _capi.make_opts(RTOL=rtol, flags=flags), fit=True)
 
 
 def staub_case(n=4, shift=0.37):

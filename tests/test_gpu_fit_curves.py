@@ -9,7 +9,7 @@ import pytest
 from metrotrpl_b200 import _capi
 from metrotrpl_b200.trial_move_evaluation import eval_trial_moves
 from tests import parity_cases as pc
-from tests.emu import fit_emu
+from tests.emu import emu
 from tests.test_fit_curves import (assert_no_side_effects, check_fit, conv_refused_case, staub_case,
                                    traps_irf_case)
 from tests.test_extrapolation_traps import traps128_problem
@@ -149,7 +149,7 @@ def test_fit_matches_host_lockstep_build(ctx):
     sel = SLOW_DECAY_STATES[:4]
     for prob, params, aux in ((prob, params[sel], aux[sel]), traps_irf_case(nx=256, n=2)[:3]):
         (ll, st, ns, cur, fit), _ = gpu_run(ctx, prob, params, aux, 0)
-        fit_e = fit_emu.loglik_batch(prob, params, aux, _capi.make_opts(RTOL=1e-7))[4]
+        fit_e = emu.loglik_batch(prob, params, aux, _capi.make_opts(RTOL=1e-7), fit=True)[4]
         np.testing.assert_array_equal(np.isnan(fit), np.isnan(fit_e))
         ok = ~np.isnan(fit)
         np.testing.assert_allclose(fit[ok], fit_e[ok], rtol=5e-7)
