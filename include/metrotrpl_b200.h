@@ -158,6 +158,15 @@ int trpl_solve_batch(trpl_handle* h, int32_t n_sets, const double* params, const
  * asking for it changes no other output. */
 int trpl_download_fit(trpl_handle* h, double* fit);
 
+/* Per-point quantiles over the parameter sets of the last run, which must have had TRPL_OPT_FIT.
+ *   q      [n_q] in [0, 1], 1 <= n_q <= TRPL_MAX_QUANTILES
+ *   quant  [n_q][n_times_total]: np.nanquantile(fit, q, axis=0, method="linear"), bit for bit
+ *   count  [n_times_total]: sets whose fitted point is not NaN (may be NULL)
+ * Only quant and count are copied to the host; the fit buffer is not.  A point no set compared
+ * (count 0) has NaN quantiles.  The fit buffer and every other result of the run stay as they are. */
+#define TRPL_MAX_QUANTILES 8
+int trpl_fit_quantiles(trpl_handle* h, int32_t n_q, const double* q, double* quant, int32_t* count);
+
 /* Split form used for device-resident timing: inputs stay in HBM between runs. */
 int trpl_upload_batch(trpl_handle* h, int32_t n_sets, const double* params, const double* aux);
 int trpl_run_resident(trpl_handle* h, const trpl_solver_opts* opts, int32_t want_curves);

@@ -31,6 +31,7 @@ ST_MAX_STEPS, ST_H_UNDERFLOW, ST_NONFINITE, ST_FLOORED, ST_NEG_FRAC, ST_NAN_LL, 
 ST_EXPLICIT = 128
 OPT_FORCE_MIN_Y, OPT_NO_LIKELIHOOD, OPT_LADDER, OPT_NO_EXPLICIT, OPT_CTA_PER_TRAJ, OPT_EXTRAPOLATION = 1, 2, 4, 8, 16, 32
 OPT_FIT = 64      # also keep the fitted curves (Context.download_fit)
+MAX_QUANTILES = 8     # TRPL_MAX_QUANTILES: levels per Context.fit_quantiles call
 
 # Defaults of the integrator.  RTOL keeps the reference's default value and meaning
 # (forward_solver.py:18).  The reference's default ATOL (1e-10 nm^-3, forward_solver.py:19) is larger
@@ -251,6 +252,7 @@ def load_library() -> C.CDLL:
     lib.trpl_run_resident.argtypes = [H, C.POINTER(SolverOpts), C.c_int32]
     lib.trpl_download_results.argtypes = [H, dp, ip, ip, dp]
     lib.trpl_download_fit.argtypes = [H, dp]
+    lib.trpl_fit_quantiles.argtypes = [H, C.c_int32, dp, dp, ip]
     lib.trpl_last_kernel_ms.argtypes = [H, C.POINTER(C.c_float)]
     lib.trpl_launch_count.argtypes = [H]
     lib.trpl_launch_count.restype = C.c_int64
@@ -422,6 +424,19 @@ class Context:
         fit = np.empty((self._n_sets, self.problem.n_times_total))
         self._check(self.lib.trpl_download_fit(self.h, _ptr(fit, C.c_double)))
         return fit
+
+    def fit_quantiles(self, q):
+        """(quant [n_q, n_times_total], count [n_times_total]) over the parameter sets of the last run,
+        which had OPT_FIT: quant equals np.nanquantile(download_fit(), q, axis=0, method="linear") bit
+        for bit, count the sets whose fitted point is not NaN.  The selection runs on the device; only
+        these two arrays are copied to the host (include/metrotrpl_b200.h, trpl_fit_quantiles)."""
+        q = np.ascontiguousarray(np.atleast_1d(q), dtype=np.float64)
+        n = self.problem.n_times_total
+        quant = np.empty((q.size, n))
+        count = np.empty(n, dtype=np.int32)
+        self._check(self.lib.trpl_fit_quantiles(self.h, int(q.size), _ptr(q, C.c_double), _ptr(quant, C.c_double),
+                                                _ptr(count, C.c_int32)))
+        return quant, count
 
     def last_kernel_ms(self) -> float:
         ms = C.c_float()

@@ -23,6 +23,7 @@
 #include "cta_trajectory.h"
 #include "extrapolation.h"
 #include "proposals.h"
+#include "fit_quantiles.h"
 
 #include "kernel_common.h"
 
@@ -169,6 +170,108 @@ __global__ void __launch_bounds__(32) trpl_fit_kernel(const KernelArgs a) {
   }
 }
 
+// trpl_fit_quantiles: exact quantiles of every point of the fit buffer over the sets of the last run,
+// by the radix select of fit_quantiles.h.  A CTA owns QT_COLS consecutive points; thread i reads point
+// i % QT_COLS of rows i / QT_COLS, + QT_ROWS, ..., so a warp reads QT_COLS consecutive doubles of each
+// of its rows (whole 32-byte sectors), QT_UNROLL rows per thread in flight.  One pass counts the
+// non-NaN values, eight passes histogram one digit each in shared memory.  Targets whose prefixes
+// agree share one histogram (all of them in the first pass), so a value lands in at most one
+// histogram per pass.  The result does not depend on the order of the atomic increments.
+constexpr int QT_COLS = 8, QT_THREADS = 256, QT_ROWS = QT_THREADS / QT_COLS, QT_UNROLL = 8;
+constexpr int QT_HSTRIDE = QT_BINS + 1;    // padding word: the per-target scans of qt_pick hit distinct banks
+
+struct QuantArgs {
+  const double* fit;      // [n_sets][n_cols]
+  double* quant;          // [n_q][n_cols]
+  int* count;             // [n_cols]
+  int n_sets, n_cols, n_q;
+  double q[TRPL_MAX_QUANTILES];
+};
+
+__global__ void __launch_bounds__(QT_THREADS) fit_quantiles_kernel(const QuantArgs a) {
+  extern __shared__ uint32_t hist[];          // [QT_COLS][2 n_q][QT_HSTRIDE]
+  __shared__ double s_q[TRPL_MAX_QUANTILES];
+  __shared__ int s_n[QT_COLS], s_nt[QT_COLS], s_rank[QT_COLS][QT_MAX_TARGETS];
+  __shared__ uint32_t s_left[QT_COLS][QT_MAX_TARGETS];
+  __shared__ uint64_t s_key[QT_COLS][QT_MAX_TARGETS];
+  const int c = threadIdx.x % QT_COLS, row0 = threadIdx.x / QT_COLS;
+  const int k = blockIdx.x * QT_COLS + c;
+  const bool live = k < a.n_cols;
+  const int T = 2 * a.n_q;
+  const double* col = a.fit + k;
+  const size_t ld = (size_t)a.n_cols;
+  if (threadIdx.x < QT_COLS) s_n[threadIdx.x] = 0;
+#pragma unroll
+  for (int j = 0; j < TRPL_MAX_QUANTILES; ++j)     // constant indices: the levels stay in parameter space
+    if (threadIdx.x == j && j < a.n_q) s_q[j] = a.q[j];
+  __syncthreads();
+  int n = 0;
+  for (int r0 = row0; live && r0 < a.n_sets; r0 += QT_ROWS * QT_UNROLL) {
+    double x[QT_UNROLL];
+#pragma unroll
+    for (int u = 0; u < QT_UNROLL; ++u) {
+      const int r = r0 + u * QT_ROWS;
+      x[u] = r < a.n_sets ? __ldg(col + r * ld) : NAN;
+    }
+#pragma unroll
+    for (int u = 0; u < QT_UNROLL; ++u) n += !isnan(x[u]);
+  }
+  atomicAdd(&s_n[c], n);
+  __syncthreads();
+  if (threadIdx.x < QT_COLS) {
+    const int cc = threadIdx.x;
+    const int nt = qt_targets(s_n[cc], a.n_q, s_q, s_rank[cc]);
+    s_nt[cc] = nt;
+    for (int t = 0; t < nt; ++t) { s_left[cc][t] = (uint32_t)s_rank[cc][t]; s_key[cc][t] = 0; }
+  }
+  for (int p = 0; p < QT_PASSES; ++p) {
+    for (int i = threadIdx.x; i < QT_COLS * T * QT_HSTRIDE; i += QT_THREADS) hist[i] = 0;
+    __syncthreads();
+    const int sh = qt_shift(p), nt = s_nt[c];
+    // the histogram a target reads: that of the first target with its prefix (ranks ascend, so the
+    // targets of one prefix are adjacent)
+    const int pc = threadIdx.x / T, pt = threadIdx.x % T;
+    const bool picks = threadIdx.x < QT_COLS * T && pt < s_nt[pc];
+    int src = pt;
+    if (picks)
+      while (src > 0 && s_key[pc][src - 1] == s_key[pc][pt]) --src;
+    uint32_t* h = hist + c * T * QT_HSTRIDE;
+    for (int r0 = row0; live && nt > 0 && r0 < a.n_sets; r0 += QT_ROWS * QT_UNROLL) {
+      double x[QT_UNROLL];
+#pragma unroll
+      for (int u = 0; u < QT_UNROLL; ++u) {
+        const int r = r0 + u * QT_ROWS;
+        x[u] = r < a.n_sets ? __ldg(col + r * ld) : NAN;
+      }
+#pragma unroll
+      for (int u = 0; u < QT_UNROLL; ++u) {
+        if (isnan(x[u])) continue;
+        const uint64_t key = qt_key(x[u]);
+        for (int t = 0; t < nt; ++t) {
+          if (t > 0 && s_key[c][t] == s_key[c][t - 1]) continue;     // not the first of its prefix
+          if (qt_match(key, s_key[c][t], p)) {
+            atomicAdd(&h[t * QT_HSTRIDE + (unsigned)((key >> sh) & (QT_BINS - 1))], 1u);
+            break;
+          }
+        }
+      }
+    }
+    __syncthreads();
+    if (picks) {
+      uint32_t left = s_left[pc][pt];
+      const unsigned d = qt_pick(hist + (pc * T + src) * QT_HSTRIDE, left);
+      s_left[pc][pt] = left;
+      s_key[pc][pt] |= (uint64_t)d << sh;
+    }
+    __syncthreads();
+  }
+  if (threadIdx.x < QT_COLS * a.n_q) {
+    const int cc = threadIdx.x / a.n_q, j = threadIdx.x % a.n_q, kk = blockIdx.x * QT_COLS + cc;
+    if (kk < a.n_cols) a.quant[(size_t)j * a.n_cols + kk] = qt_finish(s_n[cc], s_q[j], s_rank[cc], s_key[cc], s_nt[cc]);
+  }
+  if (threadIdx.x < QT_COLS && live && a.count) a.count[k] = s_n[c];
+}
+
 // Replica exchange needs each chain's likelihood at every ladder temperature summed over its
 // measurements (the reference sums ll_func[ss](T) over ss, metropolis.py:73-76): [n_sets][n_temps].
 // NaN (a failed curve) becomes -inf, as eval_trial_move's callers treat it.
@@ -244,6 +347,8 @@ struct trpl_handle {
   bool curves_valid = false;
   DevBuf<double> d_fit;
   bool fit_valid = false;
+  DevBuf<double> d_quant;
+  DevBuf<int> d_count;
   float last_ms = 0.f;
   int64_t launches = 0;
 };
@@ -698,6 +803,27 @@ int trpl_download_fit(trpl_handle* h, double* fit) {
   CU(cudaSetDevice(h->device));
   CU(cudaMemcpyAsync(fit, h->d_fit.p, sizeof(double) * (size_t)h->n_sets * h->n_times_total, cudaMemcpyDeviceToHost,
                      h->stream));
+  CU(cudaStreamSynchronize(h->stream));
+  return 0;
+}
+
+int trpl_fit_quantiles(trpl_handle* h, int32_t n_q, const double* q, double* quant, int32_t* count) {
+  if (!h || !quant) return fail("null argument");
+  if (!h->fit_valid) return fail("the last run did not produce fitted curves (run with TRPL_OPT_FIT)");
+  if (const char* why = qt_check(n_q, q)) return fail(why);
+  CU(cudaSetDevice(h->device));
+  const size_t n_cols = h->n_times_total;
+  CU(h->d_quant.reserve((size_t)n_q * n_cols));
+  CU(h->d_count.reserve(n_cols));
+  QuantArgs a{h->d_fit.p, h->d_quant.p, h->d_count.p, h->n_sets, h->n_times_total, n_q, {}};
+  for (int j = 0; j < n_q; ++j) a.q[j] = q[j];
+  const size_t smem = (size_t)QT_COLS * 2 * n_q * QT_HSTRIDE * sizeof(uint32_t);
+  CU(cudaFuncSetAttribute((const void*)fit_quantiles_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  fit_quantiles_kernel<<<(unsigned)((n_cols + QT_COLS - 1) / QT_COLS), QT_THREADS, smem, h->stream>>>(a);
+  CU(cudaGetLastError());
+  h->launches += 1;
+  CU(cudaMemcpyAsync(quant, h->d_quant.p, sizeof(double) * n_q * n_cols, cudaMemcpyDeviceToHost, h->stream));
+  if (count) CU(cudaMemcpyAsync(count, h->d_count.p, sizeof(int) * n_cols, cudaMemcpyDeviceToHost, h->stream));
   CU(cudaStreamSynchronize(h->stream));
   return 0;
 }
