@@ -97,6 +97,7 @@ extern "C" const char* trpl_emu_loglik_batch(int32_t model, int32_t n_meas, cons
   ProblemFacts pf{vals && uncs, false, irf_mom != nullptr, ladder_T ? n_ladder : 0, 0, 0};
   int max_nx = 0;
   for (int i = 0; i < n_meas; ++i) {
+    if (md[i].nx < 2 || md[i].nx > 512) return "nx must be in 2..512";
     max_nx = std::max(max_nx, md[i].nx);
     pf.max_nt = std::max(pf.max_nt, (size_t)md[i].n_t);
     if (md[i].irf_nk > 0) {
@@ -104,6 +105,10 @@ extern "C" const char* trpl_emu_loglik_batch(int32_t model, int32_t n_meas, cons
       pf.max_nrs = std::max(pf.max_nrs, (size_t)irf_resample_count(times[md[i].t_off + md[i].n_t - 1], md[i].irf_dt));
     }
   }
+  // trpl_set_problem's rule: rhs and jacobian (model.h) need the two contacts on different lanes
+  const int npl = max_nx <= 32 ? 1 : max_nx <= 64 ? 2 : 4;
+  for (int i = 0; i < n_meas; ++i)
+    if (md[i].nx <= npl) return "mixed nx: smallest nx must exceed the nodes per lane of the largest grid (1, 2 or 4)";
   bool all_full = true;
   for (int i = 0; i < n_meas; ++i) if (md[i].nx != max_nx) all_full = false;
   RunPlan p;
